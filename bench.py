@@ -364,6 +364,9 @@ def run_ours(args):
     if not args.no_cpu_baseline and rank == 0:
         digests = np.concatenate([view_digests(x.results(G.RESULT_EVIDENCE | G.RESULT_FRAGMENTS), x_part.n_bundles)
                                   for x, x_part in zip(bts, parts)]) if bts else np.zeros((0, 3), np.uint64)
+    # the event-profiled repeat above ran the same reset + bridge_all on the same inputs: the device holds the last timed step's results
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, bts, parts, per_bundle, counts)
     stage5 = stage5_gpu(ctx, bts, batch, parts, cfg, args) if not args.no_stage5 else None
     single = len(parts) == 1
     group_leg = group_bridge_gpu(ctx, bt, gp, stage5_gpu.clusters, args) if (stage5 is not None and single and cfg["mode"] == "paired") else None
@@ -1084,6 +1087,101 @@ def view_digests(res, n_bundles):
     return out
 
 
+DUMP_BYTES = 64 << 20       # --dump-outputs writes at most this much
+DUMP_SEED = 20260901        # seeds the choice of the bundles whose results are written
+DUMP_HIT_BYTES = 256        # bound on the float64 result bytes per admitted hit of the sample; the log line shows the actual value
+
+
+def _rows_index(off, rows, width=1):
+    """element indices of rows `rows` of a ragged array whose row r holds elements [off[r] * width, off[r + 1] * width)"""
+    s, n = off[rows] * width, (off[rows + 1] - off[rows]) * width
+    return np.repeat(s - np.concatenate([[0], np.cumsum(n)[:-1]]).astype(np.int64), n) + np.arange(int(n.sum()), dtype=np.int64)
+
+
+def result_arrays(res, nb, hit_off, rows):
+    """the views of agpu_batch_results(ALL) (include/aletsch_gpu.h) restricted to the bundles `rows` of the batch, as float64
+    arrays named <view>.<field>; a ragged field comes with <view>.<field>_len, its length per bundle (per cluster for the
+    cluster and bridge fields)"""
+    out = {}
+
+    def view(ptr, n):
+        return np.ctypeslib.as_array(ptr, shape=(int(n),)) if n > 0 else np.zeros(0)
+
+    def ragged(name, ptr, off, sel, width=1):
+        off = np.asarray(off, np.int64)
+        out[name] = view(ptr, int(off[-1]) * width)[_rows_index(off, sel, width)]
+        out[name + "_len"] = off[sel + 1] - off[sel]
+
+    def fixed(name, ptr, n, sel, width=1):
+        out[name] = view(ptr, n * width).reshape(-1, width)[sel].ravel() if n > 0 else np.zeros(0)
+
+    def chainset(name, v, handle_off):
+        bco = view(v.bundle_chain_off, nb + 1).astype(np.int64)
+        ch = _rows_index(bco, rows)
+        out[name + ".n_chains"] = bco[rows + 1] - bco[rows]
+        ragged(name + ".chain_val", v.chain_val, view(v.chain_off, bco[-1] + 1), ch)
+        fixed(name + ".chain_cnt", v.chain_cnt, bco[-1], ch, 3)
+        fixed(name + ".chain_grp", v.chain_grp, bco[-1], ch)
+        ragged(name + ".handle_chain", v.handle_chain, handle_off, rows)
+
+    ev, fr, gr, cl, br = res.evidence, res.fragments, res.graph, res.clusters, res.bridges
+    for f in ("lpos", "rpos", "strand"):
+        fixed("evidence." + f, getattr(ev, f), nb, rows)
+    ragged("evidence.seg", ev.seg, view(ev.seg_off, nb + 1), rows, 3)
+    ragged("evidence.splices", ev.splices, view(ev.splice_off, nb + 1), rows)
+    chainset("evidence.hcst", ev.hcst, hit_off)
+    frg_off = view(fr.frg_off, nb + 1)
+    ragged("fragments.frgs", fr.frgs, frg_off, rows, 3)
+    chainset("fragments.fcst", fr.fcst, frg_off)
+    fixed("fragments.bridged", fr.bridged, nb, rows)
+    for f, width in (("junc", 9), ("pexon", 5), ("pexon_d", 4), ("vert", 5), ("vert_d", 3), ("edge", 3), ("edge_d", 1)):
+        ragged("graph." + f, getattr(gr, f), view(getattr(gr, f.split("_")[0] + "_off"), nb + 1), rows, width)
+    fixed("graph.strand", gr.strand, nb, rows)
+    clu_off = view(cl.clu_off, nb + 1).astype(np.int64)
+    nc = int(clu_off[-1])
+    cs = _rows_index(clu_off, rows)
+    out["clusters.n_clusters"] = clu_off[rows + 1] - clu_off[rows]
+    for f, width in (("bounds", 4), ("extend", 4), ("count", 1), ("chain1", 1), ("chain2", 1)):
+        fixed("clusters." + f, getattr(cl, f), nc, cs, width)
+    ragged("clusters.frlist", cl.frlist, view(cl.frlist_off, nc + 1), cs)
+    for f in ("type", "strand", "choices", "score"):
+        fixed("bridges." + f, getattr(br, f), nc, cs)
+    ragged("bridges.chain", br.chain, view(br.chain_off, nc + 1), cs)
+    ragged("bridges.whole", br.whole, view(br.whole_off, nc + 1), cs)
+    return {k: np.asarray(v, np.float64) for k, v in out.items()}
+
+
+def dump_outputs(out_dir, bts, parts, per_bundle, counts):
+    """--dump-outputs: what the timed path (reset + bridge_all) computed in its last step, as DIR/<name>.npy (float64): the
+    batch counters, and bundle_counts plus every result view for a sample of bundles.  The sample depends on the input alone,
+    so two builds dump the same bundles: the first bundles of a permutation drawn with DUMP_SEED whose admitted hits fit
+    DUMP_BYTES at DUMP_HIT_BYTES each.  `bundle` holds the sampled bundles' indices."""
+    from aletsch_b200 import gpu as G
+    nb = sum(p.n_bundles for p in parts)
+    order = np.random.default_rng(DUMP_SEED).permutation(nb)
+    hits = np.concatenate([np.diff(p.a["bundle_hit_off"].astype(np.int64)) for p in parts])
+    rows = np.sort(order[:int(np.searchsorted(np.cumsum(hits[order]), DUMP_BYTES // DUMP_HIT_BYTES, side="right"))])
+    arrays = {"counts": np.array([counts[n] for n, _ in G.Counts._fields_], np.float64), "bundle": rows.astype(np.float64),
+              "bundle_counts": np.asarray(per_bundle, np.float64)[rows].ravel()}
+    first = 0
+    per_part = []
+    for x, part in zip(bts, parts):
+        sel = rows[(rows >= first) & (rows < first + part.n_bundles)] - first
+        first += part.n_bundles
+        per_part.append(result_arrays(x.results(G.RESULT_ALL), part.n_bundles, part.a["bundle_hit_off"].astype(np.int64), sel))
+    for name in per_part[0]:
+        arrays[name] = np.concatenate([p[name] for p in per_part])
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise SystemExit("bench.py --dump-outputs: the sampled results take %d bytes, more than %d; lower DUMP_BYTES / DUMP_HIT_BYTES"
+                         % (total, DUMP_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log("[bench] --dump-outputs: %d arrays, %.1f MB, %d of %d bundles, %.0f bytes per sampled hit -> %s" %
+        (len(arrays), total / 1e6, len(rows), nb, total / max(1, int(hits[rows].sum())), out_dir))
+
+
 def cpu_baseline(batch, cfg, threads, budget_s, gpu_bridged=None, gpu_digests=None):
     """the reference's own C++ (oracle/_ref) over a bounded sample of the same bundles (RefTimer), one untimed warm-up pass and
     then passes until the budget is used; the restatement (oracle/liboracle.so, kind "port") only if the reference build is absent"""
@@ -1238,6 +1336,8 @@ def main():
     ap.add_argument("--upload", choices=["compact", "lean"], default="compact",
                     help="host->device format of the end-to-end leg: agpu_batch_packed (default) or the lean agpu_batch_in")
     ap.add_argument("--streams", type=int, default=4, help="host threads / CUDA streams of the end-to-end pipeline")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last step to DIR/<name>.npy (float64, at most 64 MB in all)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -291,7 +291,7 @@ def test_warp_cigar_walk_on_short_reads():
               "import test_gpu_parity as T\n"
               "T.test_compact_upload_matches_full(ctx, H.SYNTH_PAIRED, 20000)\n"
               "import test_preview_insertsize as P\n"
-              "P.run_cases(ctx, chk)\n"
+              "P.run_cases(ctx, checkers.get('ref'))\n"
               "print('warp walk ok', stats['segments'])\n", "warp walk ok")
 
 

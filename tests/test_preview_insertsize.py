@@ -1,8 +1,12 @@
 """SURVEY 8f-4: previewer::infer_insertsize (meta/previewer.cc:151-304) on the C ABI against the reference's own previewer run over
 the same records through the htslib stand-in (oracle/ref_driver.cc: ref_infer_insertsize) -- its record loop, its bundle_base with
 the never-flushed interval buffer (rnacore/bundle_base.cc:106-204), build_fragments, graph_builder, graph_cluster, the histogram,
-the break at max_preview_reads and the percentiles.  CPU tier: kernel-logic build; -m gpu: the CUDA path."""
+the break at max_preview_reads and the percentiles.  CPU tier: kernel-logic build; -m gpu: the CUDA path.  Without the reference
+build CASES are compared with the profiles in tests/golden/preview_insertsize.json; its `generated_by` says where they come
+from.  `PYTHONPATH=. python tests/test_preview_insertsize.py` rewrites the file from the reference build and fails without it."""
 import ctypes as C
+import json
+import os
 
 import numpy as np
 import pytest
@@ -37,21 +41,33 @@ def reference_profile(chk, sample, n_chrom, chrom_len, op, max_reads, min_reads,
     return d
 
 
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "preview_insertsize.json")
+
+
+def stored_profiles():
+    """the stored profile of every case of CASES, in reference_profile's layout"""
+    with open(GOLDEN) as f:
+        g = json.load(f)
+    return [{"isize": np.array(d["isize"], np.int32), "isize_d": np.array(d["isize_d"], np.float64)} for d in g["cases"]]
+
+
 CASES = [(H.FR_FIRST, 1, 40000, 2000000, 100), (H.FR_FIRST, 3, 40000, 2000000, 100), (H.UNSTRANDED, 1, 40000, 2000000, 100),
          (H.UNSTRANDED, 3, 30000, 2000000, 100), (H.FR_SECOND, 2, 30000, 2000000, 100),
          (H.FR_FIRST, 2, 40000, 3000, 100),          # the break at max_preview_reads binds
          (H.FR_FIRST, 1, 2000, 2000000, 100000)]     # fewer fragments than min_preview_spliced_reads: no profile
 
 
-def run_cases(ctx, chk):
+def run_cases(ctx, chk=None):
+    """chk: the reference build's checker, or None to compare with the stored profiles"""
+    stored = None if chk is not None else stored_profiles()
     seen_skip = seen_extra = 0
-    for lt, n_chrom, templates, max_reads, min_reads in CASES:
+    for i, (lt, n_chrom, templates, max_reads, min_reads) in enumerate(CASES):
         cfg = H.default_config(H.SYNTH_PAIRED, chrom_len=2_000_000, n_chrom=n_chrom, seed=20260500 + 7 * n_chrom + lt)
         s = H.Synth(cfg).sample(0, templates, threads=4)
         gp, op = parity.params_pair(lt)
         pp = H.default_packer_params(lt)
         got = preview.infer_insertsize(ctx, s, pp, gp, max_preview_reads=max_reads, min_preview_spliced_reads=min_reads)
-        want = reference_profile(chk, s, n_chrom, 2_000_000, op, max_reads, min_reads, 10)
+        want = reference_profile(chk, s, n_chrom, 2_000_000, op, max_reads, min_reads, 10) if chk is not None else stored[i]
         where = (lt, n_chrom, templates, max_reads, min_reads)
         assert got["insert_total"] == int(want["isize"][0]), where
         if got["insert_total"] >= min_reads:
@@ -68,18 +84,15 @@ def run_cases(ctx, chk):
 
 
 def test_preview_insertsize_matches_reference(emu_lib, checkers):
-    if "ref" not in checkers:
-        pytest.skip("needs oracle/_ref/libaletsch_ref.so")
     ctx = G.Context(0, lib_path=emu_lib)
-    run_cases(ctx, checkers["ref"])
+    run_cases(ctx, checkers.get("ref"))
     ctx.close()
 
 
 def test_interval_buffer_quirk_matters(emu_lib, checkers):
     """the same run WITHOUT the coverage edits is what a clean implementation would compute; the reference's result differs from it
-    on at least one of these inputs, i.e. the quirk is observable and the edits are what reproduces it"""
-    if "ref" not in checkers:
-        pytest.skip("needs oracle/_ref/libaletsch_ref.so")
+    on at least one of these inputs, i.e. the quirk is observable and the edits are what reproduces it.  Without the reference
+    build only the second half is checked."""
     ctx = G.Context(0, lib_path=emu_lib)
     differ = 0
     for seed in range(6):
@@ -96,8 +109,9 @@ def test_interval_buffer_quirk_matters(emu_lib, checkers):
             clu_off, isize = bt.preview(gp)
             bt.free()
             res.append((H.insertsize_profile(clu_off, isize, event), isize))
-        want = reference_profile(checkers["ref"], s, 2, 1_000_000, op, 2000000, 100, 10)
-        assert res[0][0]["insert_total"] == int(want["isize"][0]), seed
+        if "ref" in checkers:
+            want = reference_profile(checkers["ref"], s, 2, 1_000_000, op, 2000000, 100, 10)
+            assert res[0][0]["insert_total"] == int(want["isize"][0]), seed
         differ += int(len(res[0][1]) != len(res[1][1]) or not np.array_equal(res[0][1], res[1][1]))
     ctx.close()
     assert differ >= 1          # the dropped blocks change graphs / clusters on this data: the quirk is observable
@@ -105,8 +119,25 @@ def test_interval_buffer_quirk_matters(emu_lib, checkers):
 
 @pytest.mark.gpu
 def test_preview_insertsize_matches_reference_gpu(checkers):
-    if "ref" not in checkers:
-        pytest.skip("needs oracle/_ref/libaletsch_ref.so")
     ctx = G.Context(0)
-    run_cases(ctx, checkers["ref"])
+    run_cases(ctx, checkers.get("ref"))
     ctx.close()
+
+
+def write_golden():
+    """record GOLDEN from the reference build's previewer (oracle/_ref); there is no other source"""
+    ref = orclib.Checker("ref")
+    cases = []
+    for lt, n_chrom, templates, max_reads, min_reads in CASES:
+        cfg = H.default_config(H.SYNTH_PAIRED, chrom_len=2_000_000, n_chrom=n_chrom, seed=20260500 + 7 * n_chrom + lt)
+        s = H.Synth(cfg).sample(0, templates, threads=4)
+        _, op = parity.params_pair(lt)
+        d = reference_profile(ref, s, n_chrom, 2_000_000, op, max_reads, min_reads, 10)
+        cases.append({"isize": [int(x) for x in d["isize"]], "isize_d": [float(x) for x in d["isize_d"]]})
+    with open(GOLDEN, "w") as f:
+        json.dump({"generated_by": "oracle/_ref/libaletsch_ref.so: ref_infer_insertsize, the reference's previewer", "cases": cases}, f, indent=1)
+        f.write("\n")
+
+
+if __name__ == "__main__":          # from the repository root: PYTHONPATH=. python tests/test_preview_insertsize.py
+    write_golden()
