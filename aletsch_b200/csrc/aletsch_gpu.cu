@@ -50,16 +50,6 @@ struct chainset_state
 	std::vector<int64_t> ext_goff_host;
 	int64_t ext_nval = 0;                 // size of the (shared) coordinate array `val` points into
 
-	void release(agpu_ctx *ctx)
-	{
-		reg_off.release(ctx); elem_slot.release(ctx); c_slot.release(ctx); val_base.release(ctx);
-		slot_word.release(ctx); key_scratch.release(ctx); key_scratch2.release(ctx);
-		slot_first.release(ctx); slot_cnt.release(ctx); slot_chain.release(ctx); n_chains.release(ctx); n_splices.release(ctx);
-		c_rep.release(ctx); c_cnt.release(ctx); c_grp.release(ctx); handle_chain.release(ctx); splices_scratch.release(ctx);
-		ext_voff.release(ctx); ext_goff.release(ctx); ext_len.release(ctx); ext_cnt3.release(ctx); ext_val.release(ctx); ext_goff_host.clear(); ext_nval = 0;
-		built = false;
-	}
-
 	chains_view view() const
 	{
 		chains_view v;
@@ -86,18 +76,6 @@ struct graph_state
 	dbuf<int32_t> e_i[3];
 	dbuf<double> e_w;
 	dbuf<int32_t> in_off, in_src, in_eid, out_off, out_dst, out_eid;
-
-	void release(agpu_ctx *ctx)
-	{
-		for(int k = 0; k < 5; k++) { ub[k].release(ctx); off[k].release(ctx); }
-		iarena.release(ctx); karena.release(ctx); n_junc.release(ctx); n_pex.release(ctx); n_edge.release(ctx);
-		for(int k = 0; k < 9; k++) j[k].release(ctx);
-		for(int k = 0; k < 6; k++) { p_i[k].release(ctx); v_i[k].release(ctx); }
-		for(int k = 0; k < 3; k++) { p_d[k].release(ctx); v_d[k].release(ctx); e_i[k].release(ctx); }
-		e_w.release(ctx);
-		in_off.release(ctx); in_src.release(ctx); in_eid.release(ctx); out_off.release(ctx); out_dst.release(ctx); out_eid.release(ctx);
-		built = false;
-	}
 
 	graph_dev dev(int *err) const
 	{
@@ -131,17 +109,70 @@ struct support_state
 	dbuf<double> vwA, vwB, ewA, ewB, abd, loss, row_val;
 	dbuf<uint8_t> aliveB;
 	std::vector<int32_t> ne_host, slot_off_host, slot_sample_host, member_group_host;
-	void release(agpu_ctx *ctx)
-	{
-		voff.release(ctx); eoff.release(ctx); row_off.release(ctx); ne.release(ctx); vl.release(ctx); vr.release(ctx); out_off.release(ctx);
-		in_off.release(ctx); in_eid.release(ctx); es.release(ctx); et.release(ctx); count.release(ctx); row_slot.release(ctx);
-		vwA.release(ctx); vwB.release(ctx); ewA.release(ctx); ewB.release(ctx); abd.release(ctx); loss.release(ctx); row_val.release(ctx);
-		aliveB.release(ctx);
-		built = false; n_groups = n_members = 0; n_vert = n_ecap = nnz = 0;
-	}
 };
 
-struct agpu_batch
+// everything the stages derive from a batch's input: agpu_batch_reset drops it by assigning a default-constructed one
+struct batch_derived
+{
+	// evidence
+	bool evidence = false;
+	dbuf<int32_t> b_lpos, b_rpos, b_covhi;
+	dbuf<uint8_t> b_strand;
+	dbuf<int64_t> b_span, cov_base;
+	int64_t ltot = 0;
+	// coverage map on border-compacted coordinates (k_evidence.h, coverage section)
+	dbuf<u32> border, wrank;
+	dbuf<int32_t> diffc, posc, covc;
+	dbuf<int64_t> bord_off, ex_s, ex_e;
+	int64_t n_bord = 0, n_extra = 0;
+	// a combined bundle's coverage sources: the borders of its members as weighted window positions (k_group.h)
+	dbuf<int64_t> pt_g;
+	dbuf<int32_t> pt_d;
+	int64_t n_pts = 0;
+	dbuf<int32_t> spl, hit_nspl, hit_bundle;
+	// insert-size preview result: fragment length per cluster (INT32_MIN: not counted)
+	dbuf<int32_t> pv_isize;
+	bool preview_built = false;
+	chainset_state hcst, fcst;
+	// segments
+	bool cov_dirty = true;
+	dbuf<int64_t> seg_off;
+	dbuf<int32_t> seg_l, seg_r, seg_c;
+	dbuf<int64_t> seg_nhead, seg_psum;     // run structure and prefix sums of len * cov over all segments (k_graph.h seg_view)
+	int64_t n_seg = 0;
+
+	// fragments / clusters / bridges live in their own headers' state structs
+	fragments_state frg;
+	graph_state gr;
+	cluster_state clu;
+	bridge_state brg;
+	bridge_entries ent;
+
+	// phasing paths (bundle_base::build_phase_set): distinct coordinate lists in element order + counts
+	bool phase_built = false;
+	int64_t n_phase = 0, n_phase_val = 0;
+	dbuf<int32_t> ph_val, ph_len, ph_cnt;
+	dbuf<int64_t> ph_off, ph_boff;
+
+	// boundary revision (identify_boundaries / remove_false_boundaries): added edges and vertex annotations, in the vertex
+	// layout of the graphs
+	bool revise_built = false;
+	dbuf<int32_t> rv_nstart, rv_nend, rv_addv, rv_leave, rv_come;
+	dbuf<double> rv_addw, rv_lratio, rv_cratio;
+	dbuf<int64_t> rv_voff;
+	int64_t rv_nvert = 0;
+
+	support_state sup;
+	// group-level re-bridge (assembler::bridge): the combined bundles of the clusters as a batch of their own (freed with
+	// agpu_batch_free)
+	agpu_batch *cb = NULL;
+	dbuf<int32_t> g_remap, g_members, g_first;
+	dbuf<int64_t> g_member_off;
+	std::vector<int32_t> g_order_host;     // members of every cluster in combine order (flattened like the input)
+	bool group_pass = false;               // cluster / bridge stages work against cb's graphs
+};
+
+struct agpu_batch : batch_derived
 {
 	int32_t nb = 0;
 	int64_t nh = 0, nc = 0;
@@ -163,67 +194,13 @@ struct agpu_batch
 
 	dbuf<int> err;
 
-	// evidence
-	bool evidence = false;
-	dbuf<int32_t> b_lpos, b_rpos, b_covhi;
-	dbuf<uint8_t> b_strand;
-	dbuf<int64_t> b_span, cov_base;
-	int64_t ltot = 0;
-	// coverage map on border-compacted coordinates (k_evidence.h, coverage section)
-	dbuf<u32> border, wrank;
-	dbuf<int32_t> diffc, posc, covc;
-	dbuf<int64_t> bord_off, ex_s, ex_e;
-	int64_t n_bord = 0, n_extra = 0;
-	// a combined bundle's coverage sources: the borders of its members as weighted window positions (k_group.h)
-	dbuf<int64_t> pt_g;
-	dbuf<int32_t> pt_d;
-	int64_t n_pts = 0;
-	dbuf<int32_t> spl, hit_nspl, hit_bundle;
 	// coverage edits of the insert-size preview (agpu_batch_coverage_edit): blocks without coverage, foreign intervals; part of the
 	// batch's INPUT (kept across agpu_batch_reset)
 	dbuf<uint16_t> cov_skip;
 	dbuf<int32_t> cov_ex_bundle, cov_ex_l, cov_ex_r, cov_ex_cnt;
 	int64_t n_cov_extra = 0;
-	// insert-size preview result: fragment length per cluster (INT32_MIN: not counted)
-	dbuf<int32_t> pv_isize;
-	bool preview_built = false;
 	bool op_warp = false;                  // this batch's evidence pass runs on the warp-per-hit CIGAR walks (long CIGARs)
-	chainset_state hcst, fcst;
-	// segments
-	bool cov_dirty = true;
-	dbuf<int64_t> seg_off;
-	dbuf<int32_t> seg_l, seg_r, seg_c;
-	dbuf<int64_t> seg_nhead, seg_psum;     // run structure and prefix sums of len * cov over all segments (k_graph.h seg_view)
-	int64_t n_seg = 0;
-
-	// fragments / clusters / bridges live in their own headers' state structs
-	fragments_state frg;
-	graph_state gr;
-	cluster_state clu;
-	bridge_state brg;
-
-	// phasing paths (bundle_base::build_phase_set): distinct coordinate lists in element order + counts
-	bool phase_built = false;
-	int64_t n_phase = 0, n_phase_val = 0;
-	dbuf<int32_t> ph_val, ph_len, ph_cnt;
-	dbuf<int64_t> ph_off, ph_boff;
-
-	// boundary revision (identify_boundaries / remove_false_boundaries): added edges and vertex annotations, in the vertex
-	// layout of the graphs
 	bool defer_check = false;
-	bool revise_built = false;
-	dbuf<int32_t> rv_nstart, rv_nend, rv_addv, rv_leave, rv_come;
-	dbuf<double> rv_addw, rv_lratio, rv_cratio;
-	dbuf<int64_t> rv_voff;
-	int64_t rv_nvert = 0;
-
-	support_state sup;
-	// group-level re-bridge (assembler::bridge): the combined bundles of the clusters as a batch of their own
-	agpu_batch *cb = NULL;
-	dbuf<int32_t> g_remap, g_members, g_first;
-	dbuf<int64_t> g_member_off;
-	std::vector<int32_t> g_order_host;     // members of every cluster in combine order (flattened like the input)
-	bool group_pass = false;               // cluster / bridge stages work against cb's graphs
 
 	// pinned result mirrors, by name: owned by the context (reused by every batch it processes); the combined bundles of a group
 	// pass are a batch of their own on the same context and prefix their names
@@ -658,26 +635,8 @@ int agpu_batch_adopt(agpu_ctx *ctx, const agpu_batch_in *in, agpu_batch **out)
 
 static void release_derived(agpu_ctx *ctx, agpu_batch *b)
 {
-	b->b_lpos.release(ctx); b->b_rpos.release(ctx); b->b_covhi.release(ctx); b->b_strand.release(ctx);
-	b->b_span.release(ctx); b->cov_base.release(ctx); b->border.release(ctx); b->wrank.release(ctx);
-	b->diffc.release(ctx); b->posc.release(ctx); b->covc.release(ctx); b->bord_off.release(ctx); b->ex_s.release(ctx); b->ex_e.release(ctx);
-	b->n_bord = 0; b->n_extra = 0;
-	b->pt_g.release(ctx); b->pt_d.release(ctx); b->n_pts = 0;
-	b->ph_val.release(ctx); b->ph_len.release(ctx); b->ph_cnt.release(ctx); b->ph_off.release(ctx); b->ph_boff.release(ctx);
-	b->phase_built = false; b->n_phase = 0; b->n_phase_val = 0;
-	b->rv_nstart.release(ctx); b->rv_nend.release(ctx); b->rv_addv.release(ctx); b->rv_leave.release(ctx); b->rv_come.release(ctx);
-	b->rv_addw.release(ctx); b->rv_lratio.release(ctx); b->rv_cratio.release(ctx); b->rv_voff.release(ctx); b->revise_built = false;
-	b->sup.release(ctx);
-	b->pv_isize.release(ctx); b->preview_built = false;
-	if(b->cb) { agpu_batch_free(ctx, b->cb); b->cb = NULL; }
-	b->g_remap.release(ctx); b->g_members.release(ctx); b->g_first.release(ctx); b->g_member_off.release(ctx); b->g_order_host.clear();
-	b->group_pass = false;
-	b->spl.release(ctx); b->hit_nspl.release(ctx); b->hit_bundle.release(ctx);
-	b->hcst.release(ctx); b->fcst.release(ctx);
-	b->seg_off.release(ctx);
-	b->seg_l.release(ctx); b->seg_r.release(ctx); b->seg_c.release(ctx); b->seg_nhead.release(ctx); b->seg_psum.release(ctx);
-	b->frg.release(ctx); b->gr.release(ctx); b->clu.release(ctx); b->brg.release(ctx); b->brg.release_entries(ctx);
-	b->evidence = false; b->cov_dirty = true; b->n_seg = 0; b->ltot = 0;
+	if(b->cb) agpu_batch_free(ctx, b->cb);
+	static_cast<batch_derived&>(*b) = batch_derived();
 }
 
 void agpu_batch_free(agpu_ctx *ctx, agpu_batch *b)
@@ -685,14 +644,9 @@ void agpu_batch_free(agpu_ctx *ctx, agpu_batch *b)
 	if(!ctx || !b) return;
 	AGPU_ENTER(ctx);
 	release_derived(ctx, b);
-	b->in_hit_off.release(ctx); b->in_pos.release(ctx); b->in_rpos.release(ctx); b->in_mpos.release(ctx); b->in_isize.release(ctx);
-	b->in_flag.release(ctx); b->in_strand.release(ctx); b->in_bstrand.release(ctx); b->in_xs.release(ctx); b->in_qid.release(ctx);
-	b->in_cigar_off.release(ctx); b->in_cigar.release(ctx);
-	b->err.release(ctx); b->order.release(ctx);
-	b->cov_skip.release(ctx); b->cov_ex_bundle.release(ctx); b->cov_ex_l.release(ctx); b->cov_ex_r.release(ctx); b->cov_ex_cnt.release(ctx);
 	stream_sync(ctx);
 	if(ctx->arena_owner == b) { ctx->arena.rewind(); ctx->arena_owner = NULL; }
-	delete b;
+	delete b;                             // the inputs: frees inside the arena's slabs are no-ops
 }
 
 int agpu_batch_reset(agpu_ctx *ctx, agpu_batch *b)
@@ -725,7 +679,6 @@ static int chainset_build(agpu_ctx *ctx, agpu_batch *b, chainset_state &cs, int6
 		TRY(lb_scan64(ctx, sz.p, nb, cs.reg_off.p));
 		TRY(d2h(ctx, &cs.n_slots, cs.reg_off.p + nb, sizeof(int64_t)));
 		TRY(stream_sync(ctx));
-		sz.release(ctx);
 	}
 	else
 	{
@@ -735,7 +688,6 @@ static int chainset_build(agpu_ctx *ctx, agpu_batch *b, chainset_state &cs, int6
 		TRY(lb_scan64(ctx, sz.p, nb, cs.reg_off.p));
 		cs.n_slots = 4 * n_elem + 2 * (int64_t)nb;
 		DEBUG_SYNC(16);
-		sz.release(ctx);
 	}
 	TRY(cs.slot_word.alloc(ctx, cs.n_slots, true));
 	TRY(cs.slot_first.alloc(ctx, cs.n_slots)); TRY(cs.slot_first.fill(ctx, 0x7f));
@@ -763,8 +715,8 @@ static int chainset_finish(agpu_ctx *ctx, agpu_batch *b, chainset_state &cs, int
 }
 
 // device-wide scans defined with stages 3-5 (abi_stages.inc)
-static int flag_rank(agpu_ctx *ctx, const int32_t *v, int64_t n, dbuf<int32_t> &tile_cnt, dbuf<int64_t> &tile_off, dbuf<int64_t> &rank, int64_t *total);
-static int value_scan(agpu_ctx *ctx, const int32_t *v, int64_t n, dbuf<int32_t> &tile_sum, dbuf<int64_t> &tile_off, dbuf<int64_t> &out, int64_t *total);
+static int flag_rank(agpu_ctx *ctx, const int32_t *v, int64_t n, dbuf<int64_t> &rank, int64_t *total);
+static int value_scan(agpu_ctx *ctx, const int32_t *v, int64_t n, dbuf<int64_t> &out, int64_t *total);
 
 // border bitmap + hits (+ the stretches of update_bridges) -> ranked borders, differences, coverage, segments
 static int coverage_scan(agpu_ctx *ctx, agpu_batch *b)
@@ -806,18 +758,14 @@ static int coverage_scan(agpu_ctx *ctx, agpu_batch *b)
 		// run structure of the segment list for the region walk of graph_builder (k_graph.h)
 		{
 			const int64_t ns = b->n_seg;
-			dbuf<int32_t> t1;
-			dbuf<int64_t> t2, hrank, heads;
-			TRY(flag_rank(ctx, s_head.p, ns, t1, t2, hrank, NULL));
+			dbuf<int64_t> hrank, heads;
+			TRY(flag_rank(ctx, s_head.p, ns, hrank, NULL));
 			TRY(heads.alloc(ctx, ns + 2)); TRY(b->seg_nhead.alloc(ctx, ns + 2));
 			LAUNCH_T(ctx, k_seg_heads, ns + 1, ns, s_head.p, hrank.p, heads.p);
 			LAUNCH_T(ctx, k_seg_nhead, ns, ns, hrank.p, heads.p, b->seg_nhead.p);
-			hrank.release(ctx); heads.release(ctx);
 		}
-		s_head.release(ctx);
 	}
 	else TRY(b->seg_psum.alloc(ctx, 2, true));
-	tot.release(ctx);
 	b->cov_dirty = false;
 	return AGPU_OK;
 }
@@ -841,7 +789,6 @@ int agpu_batch_evidence(agpu_ctx *ctx, agpu_batch *b, const agpu_params *p)
 		LAUNCH_T(ctx, k_tile_bundle, n_tiles + 1, b->h, n_tiles, tile_bundle.p);
 		LAUNCH_T(ctx, k_hit_bounds, nh, b->h, tile_bundle.p, b->b_lpos.p, b->b_rpos.p, b->b_covhi.p, npq.p, b->hit_bundle.p, b->err.p);
 		LAUNCH_T(ctx, k_bundle_finish, nb, b->h, p->library_type, b->b_lpos.p, b->b_covhi.p, npq.p, b->b_strand.p, b->b_span.p);
-		npq.release(ctx); tile_bundle.release(ctx);
 	}
 	TRY(lb_scan64(ctx, b->b_span.p, nb, b->cov_base.p));
 	b->ltot = 0;
@@ -869,7 +816,7 @@ int agpu_batch_evidence(agpu_ctx *ctx, agpu_batch *b, const agpu_params *p)
 	chainset_state &cs = b->hcst;
 	cs.val = b->spl.p; cs.voff32 = b->h.cigar_off; cs.voff64 = NULL; cs.elem_len = b->hit_nspl.p;
 	TRY(chainset_build(ctx, b, cs, nh, b->h.bundle_hit_off, n_spliced.p));
-	n_spliced.release(ctx);
+	n_spliced.release();
 	LAUNCH_T(ctx, k_hcst_insert, nh, b->h, b->hit_nspl.p, b->hit_bundle.p, b->spl.p, cs.reg_off.p, cs.slot_word.p,
 			cs.slot_first.p, cs.slot_cnt.p, cs.elem_slot.p, b->err.p);
 	TRY(cs.val_base.alloc(ctx, nb + 1));
@@ -888,7 +835,7 @@ int agpu_batch_graph(agpu_ctx *ctx, agpu_batch *b, const agpu_params *p)
 	if(!b->evidence) return AGPU_ERR_ARG;
 	if(b->cov_dirty) TRY(coverage_scan(ctx, b));
 	graph_state &gs = b->gr;
-	gs.release(ctx);
+	gs = graph_state();
 	int nb = b->nb;
 	graph_in in;
 	in.n = nb; in.lpos = b->b_lpos.p; in.rpos = b->b_rpos.p; in.strand = b->b_strand.p;

@@ -1140,7 +1140,6 @@ KERNEL k_scatter_handle(int64_t n_ent, int32_t n_bundles, const int64_t *ent_bof
 struct bridge_state
 {
 	bool built = false;
-	int64_t n_chain_val = 0;
 	agpu::dbuf<int32_t> vp1, vp2, pier_of, n_piers, n_groups, p_bs, p_bt, p_group, g_k1, g_k2, g_first, g_last, maxin;
 	agpu::dbuf<int64_t> g_rows, g_row_off, g_cand_need, g_cand_off, p_path_need, p_path_off;
 	agpu::dbuf<int32_t> t_cnt, t_len, t_tr1, t_tr2, t_stack, cand, cand_idx, p_nbr, br_len, br_clen, br_stack, br_order, paths, chains;
@@ -1149,37 +1148,16 @@ struct bridge_state
 	agpu::dbuf<int32_t> o_type, o_strand, o_choices, o_clen, o_wlen, o_chain, o_whole;
 	agpu::dbuf<double> o_score;
 	agpu::dbuf<int64_t> o_coff, o_woff;
-	agpu::dbuf<int32_t> tile_cnt;
-	agpu::dbuf<int64_t> tile_off;
 	int64_t n_clu = 0, n_cval = 0, n_wval = 0;
-	// update / fcst entries (all rounds)
-	agpu::dbuf<int32_t> acc_cnt, ent_cnt;
-	agpu::dbuf<int64_t> ent_off;
+	bool updated = false;
+};
+
+// update / fcst entries of all update rounds: a re-bridge (group pass) starts a new bridge_state and appends to these
+struct bridge_entries
+{
 	agpu::dbuf<int32_t> ent_frag, ent_xs, ent_len, fc_val, frag_chain;
 	agpu::dbuf<int64_t> ent_voff, ent_boff;
-	int64_t n_ent = 0;
-	bool updated = false;
-
-	void release(agpu_ctx *ctx)
-	{
-		vp1.release(ctx); vp2.release(ctx); pier_of.release(ctx); n_piers.release(ctx); n_groups.release(ctx); p_bs.release(ctx); p_bt.release(ctx);
-		p_group.release(ctx); g_k1.release(ctx); g_k2.release(ctx); g_first.release(ctx); g_last.release(ctx); maxin.release(ctx);
-		g_rows.release(ctx); g_row_off.release(ctx); g_cand_need.release(ctx); g_cand_off.release(ctx); p_path_need.release(ctx); p_path_off.release(ctx);
-		t_cnt.release(ctx); t_len.release(ctx); t_tr1.release(ctx); t_tr2.release(ctx); t_stack.release(ctx); cand.release(ctx); cand_idx.release(ctx);
-		p_nbr.release(ctx); br_len.release(ctx); br_clen.release(ctx); br_stack.release(ctx); br_order.release(ctx); paths.release(ctx); chains.release(ctx);
-		key_scratch.release(ctx);
-		o_type.release(ctx); o_strand.release(ctx); o_choices.release(ctx); o_clen.release(ctx); o_wlen.release(ctx); o_chain.release(ctx); o_whole.release(ctx);
-		o_score.release(ctx); o_coff.release(ctx); o_woff.release(ctx); tile_cnt.release(ctx); tile_off.release(ctx);
-		acc_cnt.release(ctx); ent_cnt.release(ctx); ent_off.release(ctx);
-		built = false; updated = false;
-	}
-
-	void release_entries(agpu_ctx *ctx)
-	{
-		ent_frag.release(ctx); ent_xs.release(ctx); ent_len.release(ctx); fc_val.release(ctx); frag_chain.release(ctx);
-		ent_voff.release(ctx); ent_boff.release(ctx);
-		n_ent = 0; n_chain_val = 0;
-	}
+	int64_t n_ent = 0, n_chain_val = 0;
 };
 
 #endif

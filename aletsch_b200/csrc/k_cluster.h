@@ -896,27 +896,12 @@ struct cluster_state
 	agpu::dbuf<int32_t> f_ok, m_a1, m_a2, f_next, leader, leader_size;
 	agpu::dbuf<agpu::u64> f_hash, slot_word, elems;
 	agpu::dbuf<int64_t> f_slot, reg_off, member_off, member_boff, crank, clu_off;
-	agpu::dbuf<int32_t> slot_min, slot_n, slot_head, members, cflag, tile_cnt, n_big, big_list, part_scratch;
-	agpu::dbuf<int64_t> tile_off, grank;
+	agpu::dbuf<int32_t> slot_min, slot_n, slot_head, members, cflag, n_big, big_list, part_scratch;
 	// clusters
 	int64_t n_mem = 0, n_clu = 0;
 	agpu::dbuf<int32_t> c_bounds, c_extend, c_count, c_chain1, c_chain2, c_bundle;
 	agpu::dbuf<int64_t> c_fr_begin;
 	std::vector<int64_t> clu_off_host;
-
-	void release(agpu_ctx *ctx)
-	{
-		cp_valid.release(ctx); cp_mono.release(ctx); cp_first.release(ctx); cp_last.release(ctx); cp_nruns.release(ctx); cp_runs.release(ctx);
-		f_ok.release(ctx); m_a1.release(ctx); m_a2.release(ctx); f_next.release(ctx); leader.release(ctx); leader_size.release(ctx);
-		f_hash.release(ctx); slot_word.release(ctx); elems.release(ctx); f_slot.release(ctx); reg_off.release(ctx); member_off.release(ctx);
-		member_boff.release(ctx); crank.release(ctx); clu_off.release(ctx);
-		slot_min.release(ctx); slot_n.release(ctx); slot_head.release(ctx); members.release(ctx); cflag.release(ctx); tile_cnt.release(ctx);
-		n_big.release(ctx); big_list.release(ctx); part_scratch.release(ctx);
-		tile_off.release(ctx); grank.release(ctx);
-		c_bounds.release(ctx); c_extend.release(ctx); c_count.release(ctx); c_chain1.release(ctx); c_chain2.release(ctx); c_bundle.release(ctx);
-		c_fr_begin.release(ctx);
-		built = false; n_mem = 0; n_clu = 0;
-	}
 
 	agpu::chain_paths paths()
 	{

@@ -252,19 +252,11 @@ KERNEL k_gather_i64(int64_t n, const int64_t *idx, const int64_t *src, int64_t *
 struct fragments_state
 {
 	bool built = false;
-	agpu::dbuf<int32_t> mate, tile_cnt;
-	agpu::dbuf<int64_t> tile_off, rank, frg_off;
+	agpu::dbuf<int32_t> mate;
+	agpu::dbuf<int64_t> rank, frg_off;
 	agpu::dbuf<int32_t> f_h1, f_h2, f_type, f_bundle, bridged;
 	int64_t n_frg = 0;
 	std::vector<int64_t> frg_off_host;
-
-	void release(agpu_ctx *ctx)
-	{
-		mate.release(ctx); tile_cnt.release(ctx);
-		tile_off.release(ctx); rank.release(ctx); frg_off.release(ctx);
-		f_h1.release(ctx); f_h2.release(ctx); f_type.release(ctx); f_bundle.release(ctx); bridged.release(ctx);
-		built = false; n_frg = 0;
-	}
 };
 
 #endif

@@ -336,19 +336,32 @@ inline void lb_destroy(agpu_ctx *ctx)
 	emu_launch(true, kern, g_, 256, lc_, __VA_ARGS__); (ctx)->launches++; } } while(0)
 #endif
 
-// stream-ordered device array
+// stream-ordered device array: owns its allocation and frees it (on the stream of the context it came from) when it goes.
+// Never give one static storage duration: its destructor would run after the CUDA context is gone.
 template<typename T> struct dbuf
 {
 	T *p = NULL;
 	size_t n = 0;
-	int alloc(agpu_ctx *ctx, size_t count, bool zero = false)
+	agpu_ctx *ctx = NULL;
+	dbuf() = default;
+	dbuf(const dbuf &) = delete;
+	dbuf &operator=(const dbuf &) = delete;
+	dbuf(dbuf &&o) : p(o.p), n(o.n), ctx(o.ctx) { o.p = NULL; o.n = 0; }
+	dbuf &operator=(dbuf &&o)
 	{
-		release(ctx);
-		n = count;
-		return dev_alloc_bytes(ctx, (void**)&p, count * sizeof(T), zero);
+		if(this != &o) { release(); p = o.p; n = o.n; ctx = o.ctx; o.p = NULL; o.n = 0; }
+		return *this;
 	}
-	void release(agpu_ctx *ctx) { if(p) dev_free_bytes(ctx, p); p = NULL; n = 0; }
-	int fill(agpu_ctx *ctx, int byte) { return dev_fill(ctx, p, byte, n * sizeof(T)); }
+	~dbuf() { release(); }
+	int alloc(agpu_ctx *c, size_t count, bool zero = false)
+	{
+		release();
+		ctx = c;
+		n = count;
+		return dev_alloc_bytes(c, (void**)&p, count * sizeof(T), zero);
+	}
+	void release() { if(p) dev_free_bytes(ctx, p); p = NULL; n = 0; }
+	int fill(agpu_ctx *c, int byte) { return dev_fill(c, p, byte, n * sizeof(T)); }
 };
 
 } // namespace agpu
