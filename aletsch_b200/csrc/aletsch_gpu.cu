@@ -122,7 +122,7 @@ struct batch_derived
 	int64_t ltot = 0;
 	// coverage map on border-compacted coordinates (k_evidence.h, coverage section)
 	dbuf<u32> border, wrank;
-	dbuf<int32_t> diffc, posc, covc;
+	dbuf<int32_t> diffc, posc;
 	dbuf<int64_t> bord_off, ex_s, ex_e;
 	int64_t n_bord = 0, n_extra = 0;
 	// a combined bundle's coverage sources: the borders of its members as weighted window positions (k_group.h)
@@ -139,7 +139,9 @@ struct batch_derived
 	dbuf<int64_t> seg_off;
 	dbuf<int32_t> seg_l, seg_r, seg_c;
 	dbuf<int64_t> seg_nhead, seg_psum;     // run structure and prefix sums of len * cov over all segments (k_graph.h seg_view)
+	dbuf<int64_t> cov_tot;                 // [0] borders, [1] segments
 	int64_t n_seg = 0;
+	bool n_seg_on_dev = false;             // n_seg is still to be read back from cov_tot (seg_count)
 
 	// fragments / clusters / bridges live in their own headers' state structs
 	fragments_state frg;
@@ -714,59 +716,59 @@ static int chainset_finish(agpu_ctx *ctx, agpu_batch *b, chainset_state &cs, int
 	return AGPU_OK;
 }
 
-// device-wide scans defined with stages 3-5 (abi_stages.inc)
-static int flag_rank(agpu_ctx *ctx, const int32_t *v, int64_t n, dbuf<int64_t> &rank, int64_t *total);
-static int value_scan(agpu_ctx *ctx, const int32_t *v, int64_t n, dbuf<int64_t> &out, int64_t *total);
-
-// border bitmap + hits (+ the stretches of update_bridges) -> ranked borders, differences, coverage, segments
+// border bitmap + hits (+ the stretches of update_bridges) -> ranked borders, differences, coverage, segments.  One stream drain:
+// the border count, which sizes the per-border arrays.  The segment count stays on the device (cov_tot[1]) and is read back
+// with the next read-back that needs it (seg_count).
 static int coverage_scan(agpu_ctx *ctx, agpu_batch *b)
 {
 	const int nb = b->nb;
 	TRY(b->seg_off.alloc(ctx, nb + 2, true));
-	b->n_seg = 0; b->n_bord = 0;
+	b->n_seg = 0; b->n_bord = 0; b->n_seg_on_dev = false;
 	const int64_t nw = b->ltot / 32;
-	dbuf<int64_t> tot;
-	TRY(tot.alloc(ctx, 4, true));
+	TRY(b->cov_tot.alloc(ctx, 4, true));
 	if(nw > 0)
 	{
 		// rank the borders: one look-back pass over the bitmap words
 		TRY(b->wrank.alloc(ctx, nw + 2));
-		LAUNCH_LB(ctx, k_lb_bord_rank, (nw + 1 + LB_TILE - 1) / LB_TILE, b->border.p, nw, b->wrank.p, tot.p);
-		TRY(d2h(ctx, &b->n_bord, tot.p, sizeof(int64_t)));
+		LAUNCH_LB(ctx, k_lb_bord_rank, (nw + 1 + LB_TILE - 1) / LB_TILE, b->border.p, nw, b->wrank.p, b->cov_tot.p);
+		TRY(d2h(ctx, &b->n_bord, b->cov_tot.p, sizeof(int64_t)));
 		TRY(stream_sync(ctx));
 	}
 	const int64_t n = b->n_bord;
 	TRY(b->seg_l.alloc(ctx, n + 1)); TRY(b->seg_r.alloc(ctx, n + 1)); TRY(b->seg_c.alloc(ctx, n + 1));
 	if(n > 0)
 	{
-		TRY(b->diffc.alloc(ctx, n + 1, true)); TRY(b->posc.alloc(ctx, n + 1)); TRY(b->covc.alloc(ctx, n + 1));
-		TRY(b->bord_off.alloc(ctx, nb + 2));
-		LAUNCH_T(ctx, k_bord_off, nb + 1, nb, b->cov_base.p, b->wrank.p, b->bord_off.p);
-		LAUNCH_T(ctx, k_bord_positions, nw, nw, b->border.p, b->wrank.p, nb, b->cov_base.p, b->b_lpos.p, b->posc.p);
+		TRY(b->diffc.alloc(ctx, n + 1, true)); TRY(b->posc.alloc(ctx, n + 1));
+		const int64_t n_tiles = (n + 1 + LB_TILE - 1) / LB_TILE;      // tiles of k_lb_cov_segments
+		dbuf<int32_t> tile_b0;
+		TRY(b->bord_off.alloc(ctx, nb + 2)); TRY(tile_b0.alloc(ctx, n_tiles + 1));
+		LAUNCH_T(ctx, k_bord_off, nb + 1, nb, b->cov_base.p, b->wrank.p, b->bord_off.p, n_tiles, tile_b0.p);
+		LAUNCH_B(ctx, k_bord_positions, (nw + LB_TILE - 1) / LB_TILE, 256, nw, b->border.p, b->wrank.p, nb, b->cov_base.p, b->b_lpos.p, b->posc.p);
 		if(b->op_warp) LAUNCH_B(ctx, k_cov_add_warp, CW_GRID(ctx, b->nh), CW_WARPS * CW_WS, b->h, b->hit_bundle.p, b->b_lpos.p, b->cov_base.p, b->border.p, b->wrank.p, b->diffc.p, b->cov_skip.p);
 		else LAUNCH_T(ctx, k_cov_add, HQ_THREADS(b->nh), b->h, b->hit_bundle.p, b->b_lpos.p, b->cov_base.p, b->border.p, b->wrank.p, b->diffc.p, b->cov_skip.p);
 		LAUNCH_T(ctx, k_cov_add_extra, b->n_extra, b->n_extra, b->ex_s.p, b->ex_e.p, b->border.p, b->wrank.p, b->diffc.p);
 		LAUNCH_T(ctx, k_cov_add_points, b->n_pts, b->n_pts, b->pt_g.p, b->pt_d.p, b->border.p, b->wrank.p, b->diffc.p);
 		// coverage = prefix sum of the differences; segments = borders with positive coverage; prefix sums of len * cov:
-		// one launch, three chained look-backs
-		dbuf<int32_t> s_head;
-		TRY(s_head.alloc(ctx, n + 1)); TRY(b->seg_psum.alloc(ctx, n + 2));
-		LAUNCH_LB(ctx, k_lb_cov_segments, (n + 1 + LB_TILE - 1) / LB_TILE, b->diffc.p, b->posc.p, n, nb, b->bord_off.p, b->covc.p,
-				b->seg_l.p, b->seg_r.p, b->seg_c.p, b->seg_off.p, s_head.p, b->seg_psum.p, tot.p + 1);
-		TRY(d2h(ctx, &b->n_seg, tot.p + 1, sizeof(int64_t)));
-		TRY(stream_sync(ctx));
-		// run structure of the segment list for the region walk of graph_builder (k_graph.h)
-		{
-			const int64_t ns = b->n_seg;
-			dbuf<int64_t> hrank, heads;
-			TRY(flag_rank(ctx, s_head.p, ns, hrank, NULL));
-			TRY(heads.alloc(ctx, ns + 2)); TRY(b->seg_nhead.alloc(ctx, ns + 2));
-			LAUNCH_T(ctx, k_seg_heads, ns + 1, ns, s_head.p, hrank.p, heads.p);
-			LAUNCH_T(ctx, k_seg_nhead, ns, ns, hrank.p, heads.p, b->seg_nhead.p);
-		}
+		// one launch, three chained look-backs.  Then the run structure.  Both are sized by the border count, an upper bound of the
+		// segment count
+		dbuf<uint8_t> s_head;
+		TRY(s_head.alloc(ctx, n + 1)); TRY(b->seg_psum.alloc(ctx, n + 2)); TRY(b->seg_nhead.alloc(ctx, n + 2));
+		LAUNCH_LB(ctx, k_lb_cov_segments, n_tiles, b->diffc.p, b->posc.p, n, nb, b->bord_off.p, tile_b0.p,
+				b->seg_l.p, b->seg_r.p, b->seg_c.p, b->seg_off.p, s_head.p, b->seg_psum.p, b->cov_tot.p + 1);
+		LAUNCH_B(ctx, k_seg_nhead, (n + LB_TILE - 1) / LB_TILE, LB_THREADS, n, s_head.p, b->cov_tot.p + 1, b->seg_nhead.p);
+		b->n_seg_on_dev = true;
 	}
 	else TRY(b->seg_psum.alloc(ctx, 2, true));
 	b->cov_dirty = false;
+	return AGPU_OK;
+}
+
+// queue the copy of the segment count coverage_scan left on the device; b->n_seg holds it after the caller's next stream drain
+static int seg_count(agpu_ctx *ctx, agpu_batch *b)
+{
+	if(!b->n_seg_on_dev) return AGPU_OK;
+	TRY(d2h(ctx, &b->n_seg, b->cov_tot.p + 1, sizeof(int64_t)));
+	b->n_seg_on_dev = false;
 	return AGPU_OK;
 }
 

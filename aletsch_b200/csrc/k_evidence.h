@@ -473,41 +473,16 @@ KERNEL k_gather_off(int64_t n, const int64_t *idx, const u32 *src, int64_t *out)
 //   wrank[L/32+1]  exclusive prefix popcount of the bitmap words: rank of a position among the borders
 //   diffc[NB]      difference array indexed by border rank;   posc[NB] genomic coordinate of every border
 // A bundle's differences sum to 0, so ONE device-wide prefix sum over diffc yields every bundle's coverage, and one
-// device-wide rank of (coverage > 0) compacts the segments: seg i = (posc[i], posc[i + 1], cov[i]).
+// device-wide rank of (coverage > 0) compacts the segments: seg i = (posc[i], posc[i + 1], coverage right of border i).
+// Launches (coverage_scan): k_lb_bord_rank (wrank) -- border count read back, it sizes the per-border arrays -- k_bord_off,
+// k_bord_positions (posc), the k_cov_add* kernels (diffc), k_lb_cov_segments (coverage, segments, seg_psum, seg_off, run
+// heads; the coverage itself is not stored), k_seg_nhead (run structure).  The segment count stays on the device.
 
 // rank of global window position g among the borders (g itself must be a border)
 DEV int64_t border_rank(const u32 *border, const u32 *wrank, int64_t g)
 {
 	u32 w = border[g >> 5];
 	return (int64_t)wrank[g >> 5] + __popc(w & ((1u << (g & 31)) - 1u));
-}
-
-// genomic coordinate of every border; one thread per bitmap word
-KERNEL k_bord_positions(int64_t n_words, const u32 *border, const u32 *wrank, int32_t n_bundles, const int64_t *cov_base,
-		const int32_t *b_lpos, int32_t *posc)
-{
-	int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-	if(w >= n_words) return;
-	u32 bits = border[w];
-	if(!bits) return;
-	int64_t g0 = w << 5;
-	int b = find_segment(cov_base, n_bundles, g0);
-	int32_t p0 = (int32_t)(g0 - cov_base[b]) + b_lpos[b];
-	int64_t o = wrank[w];
-	while(bits)
-	{
-		int k = __ffs((int)bits) - 1;
-		bits &= bits - 1;
-		posc[o++] = p0 + k;
-	}
-}
-
-// bord_off[b] = rank of the first border of bundle b's window (bord_off[NB] = total)
-KERNEL k_bord_off(int32_t nb, const int64_t *cov_base, const u32 *wrank, int64_t *bord_off)
-{
-	int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-	if(i > nb) return;
-	bord_off[i] = (int64_t)wrank[cov_base[i] >> 5];
 }
 
 // one thread per hit: +1 at the start and -1 at the end of every BAM_CMATCH block (bundle_base::add_intervals,
@@ -573,23 +548,6 @@ KERNEL k_cov_add_extra(int64_t n, const int64_t *ex_s, const int64_t *ex_e, cons
 	atomicAdd(&diffc[border_rank(border, wrank, ex_e[i])], -1);
 }
 
-// heads[k] = index of the k-th run-opening segment (heads[total] = n)
-KERNEL k_seg_heads(int64_t n, const int32_t *seg_head, const int64_t *hrank, int64_t *heads)
-{
-	int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-	if(i > n) return;
-	if(i == n) { heads[hrank[n]] = n; return; }
-	if(seg_head[i] >= 0) heads[hrank[i]] = i;
-}
-
-// nhead[i] = first run-opening segment after i
-KERNEL k_seg_nhead(int64_t n, const int64_t *hrank, const int64_t *heads, int64_t *nhead)
-{
-	int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-	if(i >= n) return;
-	nhead[i] = heads[hrank[i + 1]];
-}
-
 // ---- single-pass versions (decoupled look-back, lookback.h) of the coverage scans ------------------------------------------
 
 // wrank[w] = number of borders before bitmap word w (wrank[n_words] = total); *total gets the number of borders
@@ -617,16 +575,74 @@ KERNEL k_lb_bord_rank(lb_ctl c, const u32 *border, int64_t n_words, u32 *wrank, 
 	}
 }
 
+// bord_off[b] = rank of the first border of bundle b's window (bord_off[NB] = total); tile_b0[k] = first bundle whose first border
+// has rank >= k * LB_TILE, for the tiles of k_lb_cov_segments (a bisection of bord_off per tile there sat on every tile's path)
+KERNEL k_bord_off(int32_t nb, const int64_t *cov_base, const u32 *wrank, int64_t *bord_off, int64_t n_tiles, int32_t *tile_b0)
+{
+	int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+	if(i > nb) return;
+	const int64_t cur = (int64_t)wrank[cov_base[i] >> 5], prev = i > 0 ? (int64_t)wrank[cov_base[i - 1] >> 5] : -1;
+	bord_off[i] = cur;
+	for(int64_t k = (prev + LB_TILE) / LB_TILE; k <= cur / LB_TILE && k < n_tiles; k++) tile_b0[k] = (int32_t)i;
+}
+
+// genomic coordinate of every border: posc[rank] (posc is sized by the border count, so this runs after it is read back).
+// Tiles of LB_TILE words; bundle windows start at multiples of COV_ALIGN positions, so each group of COV_ALIGN / 32 words belongs
+// to one bundle: two bisections per tile find the tile's bundles, and every group looks its bundle up among those.
+#define BP_GROUP (COV_ALIGN / 32)
+KERNEL k_bord_positions(int64_t n_words, const u32 *border, const u32 *wrank, int32_t n_bundles, const int64_t *cov_base,
+		const int32_t *b_lpos, int32_t *posc)
+{
+	SHARED long long s_delta[LB_TILE / BP_GROUP];      // per group of words: b_lpos - cov_base of its bundle
+	SHARED int s_b[2];
+	const int64_t n_tiles = (n_words + LB_TILE - 1) / LB_TILE;
+	for(int64_t t = blockIdx.x; t < n_tiles; t += gridDim.x)
+	{
+		const int64_t g0 = t * LB_TILE;
+		if(threadIdx.x == 0)
+		{
+			const int64_t last = (g0 + LB_TILE < n_words ? g0 + LB_TILE : n_words) - 1;
+			s_b[0] = find_segment(cov_base, n_bundles, g0 << 5);
+			s_b[1] = find_segment(cov_base, n_bundles, last << 5);
+		}
+		BLOCK_SYNC();
+		const int b0 = s_b[0], b1 = s_b[1];
+		for(int k = threadIdx.x; k < LB_TILE / BP_GROUP; k += blockDim.x)
+		{
+			const int b = b0 + find_segment(cov_base + b0, b1 - b0, (g0 + (int64_t)k * BP_GROUP) << 5);
+			s_delta[k] = b < n_bundles ? (long long)b_lpos[b] - cov_base[b] : 0;
+		}
+		BLOCK_SYNC();
+		for(int i = threadIdx.x; i < LB_TILE; i += blockDim.x)
+		{
+			const int64_t w = g0 + i;
+			u32 x = w < n_words ? border[w] : 0u;
+			if(!x) continue;
+			const int32_t p0 = (int32_t)((w << 5) + s_delta[i / BP_GROUP]);
+			int64_t o = wrank[w];
+			while(x)
+			{
+				const int k = __ffs((int)x) - 1;
+				x &= x - 1;
+				posc[o++] = p0 + k;
+			}
+		}
+		BLOCK_SYNC();
+	}
+}
+
 // differences -> coverage -> segments, one launch.  Three chained look-backs per tile of borders:
-//   chain 0: sum of the differences        -> cov[i] = coverage right of border i
-//   chain 1: number of borders with cov > 0 -> position of every segment in the compact list
+//   chain 0: sum of the differences        -> coverage right of every border
+//   chain 1: number of borders with coverage > 0 -> position of every segment in the compact list
 //   chain 2: sum of the products (r - l) * c of the tile's segments, int32 wrap-around arithmetic -> seg_psum
-// Outputs: the segments in order -- border i with cov[i] > 0 opens [posc[i], posc[i + 1]) with value cov[i] -- as seg_l / seg_r /
-// seg_c; seg_head[o] = 0 if segment o does not touch its predecessor (it opens a run of region::build_join_interval_map), else -1;
-// seg_psum[o] = sum of the products (r - l) * c, int32 arithmetic (the summands of compute_sum_overlap), of the segments before o
-// (seg_psum[n_seg] = total); seg_off[b] = number of segments before the first border of bundle b; *n_seg.
-KERNEL k_lb_cov_segments(lb_ctl c, const int32_t *diffc, const int32_t *posc, int64_t n, int32_t n_bundles, const int64_t *bord_off,
-		int32_t *cov, int32_t *seg_l, int32_t *seg_r, int32_t *seg_c, int64_t *seg_off, int32_t *seg_head, int64_t *seg_psum, int64_t *n_seg)
+// Outputs: the segments in order -- border i with coverage c > 0 opens [posc[i], posc[i + 1]) with value c -- as seg_l / seg_r /
+// seg_c; seg_head[o] = 1 if segment o does not touch its predecessor (it opens a run of region::build_join_interval_map), else 0;
+// seg_psum[o] = the int64 sum of the int32-wrapped product totals of the tiles before o's tile, plus the int32-wrapped sum of the
+// products of the segments before o in its tile (seg_psum[n_seg] = total; only differences of nearby entries are read, cut to
+// int32: the summands of compute_sum_overlap); seg_off[b] = number of segments before the first border of bundle b; *n_seg.
+// Capped at 40 registers for six CTAs per SM: a tile spends most of its time waiting on look-backs, and resident tiles hide that.
+KERNEL_OCC(6) k_lb_cov_segments(lb_ctl c, const int32_t *diffc, const int32_t *posc, int64_t n, int32_t n_bundles, const int64_t *bord_off,
+		const int32_t *tile_b0, int32_t *seg_l, int32_t *seg_r, int32_t *seg_c, int64_t *seg_off, uint8_t *seg_head, int64_t *seg_psum, int64_t *n_seg)
 {
 	SHARED16 int f[LB_TILE + 1];     // local prefix of the differences, then of the segment flags
 	SHARED int cv[LB_TILE + 1];      // coverage of the tile's borders; cv[LB_TILE]: coverage of the border before the tile
@@ -647,9 +663,7 @@ KERNEL k_lb_cov_segments(lb_ctl c, const int32_t *diffc, const int32_t *posc, in
 		for(int i = threadIdx.x; i < LB_TILE; i += blockDim.x)
 		{
 			const int64_t g = g0 + i;
-			const int cc = g < n ? pre + f[i] + diffc[g] : 0;
-			cv[i] = cc;
-			if(g < n) cov[g] = cc;
+			cv[i] = g < n ? pre + f[i] + diffc[g] : 0;
 		}
 		if(threadIdx.x == 0) cv[LB_TILE] = pre;      // coverage right of border g0 - 1 = sum of all differences before the tile
 		BLOCK_SYNC();
@@ -668,10 +682,9 @@ KERNEL k_lb_cov_segments(lb_ctl c, const int32_t *diffc, const int32_t *posc, in
 		}
 		BLOCK_SYNC();
 		const int cnt = block_excl_scan(f, LB_TILE);
-		if(threadIdx.x == 0) f[LB_TILE] = cnt;
 		const int psum = block_excl_scan(pr, LB_TILE);
-		const int64_t o0 = lb_tile_prefix(c, 1, t, cnt);
-		const int64_t q0 = lb_tile_prefix(c, 2, t, psum);
+		int64_t o0, q0;
+		lb_tile_prefix2(c, 1, 2, t, cnt, psum, &o0, &q0);
 		for(int i = threadIdx.x; i < LB_TILE; i += blockDim.x)
 		{
 			const int64_t g = g0 + i;
@@ -680,16 +693,80 @@ KERNEL k_lb_cov_segments(lb_ctl c, const int32_t *diffc, const int32_t *posc, in
 			const int32_t pl = posc[g], prr = g + 1 < n ? posc[g + 1] : posc[g];
 			seg_l[o] = pl; seg_r[o] = prr; seg_c[o] = cv[i];
 			const int before = i > 0 ? cv[i - 1] : cv[LB_TILE];
-			seg_head[o] = (g > 0 && before > 0) ? -1 : 0;
+			seg_head[o] = (g > 0 && before > 0) ? 0 : 1;
 			seg_psum[o] = q0 + pr[i];
 		}
 		const bool last = t == n_tiles - 1;
 		if(last && threadIdx.x == 0) { seg_psum[o0 + cnt] = q0 + psum; *n_seg = o0 + cnt; }
 		// bundles whose first border falls into this tile (the last tile also owns rank n)
 		const int64_t hi = last ? n + 1 : g0 + LB_TILE;
-		const int b0 = lower_bound_idx(bord_off, n_bundles + 1, g0);
-		for(int b = b0 + (int)threadIdx.x; b <= n_bundles && bord_off[b] < hi; b += blockDim.x)
+		for(int b = tile_b0[t] + (int)threadIdx.x; b <= n_bundles && bord_off[b] < hi; b += blockDim.x)
 			seg_off[b] = o0 + f[bord_off[b] - g0];
+		BLOCK_SYNC();
+	}
+}
+
+// seg_nhead[o] = first segment after o that opens a run (n_seg if none), for the region walk of k_graph.h.  Tile t holds the
+// segments n_seg - 1 - t * LB_TILE downwards (element k: segment top - k), so the next head of an element is the nearest head among
+// the elements before it: an exclusive maximum scan of the heads' element indices.  What lies after the tile is found by reading
+// the run heads that follow it until one is set -- runs are short (a run ends where the coverage drops to zero, at the latest at
+// the end of the bundle), so tiles do not wait for each other.  The segment count stays on the device: the launch is sized by the
+// border count, and tiles past the segments return at once.
+#ifndef AGPU_EMU
+#define NH_LANES 32
+#else
+#define NH_LANES 1               // kernel-logic build: one thread per CTA
+#endif
+KERNEL k_seg_nhead(int64_t n_bord, const uint8_t *seg_head, const int64_t *n_seg, int64_t *nhead)
+{
+	SHARED int s_tot[LB_ROW_TOTALS];
+	SHARED long long s_after;
+	const int64_t ns = *n_seg;
+	const int64_t n_tiles = (n_bord + LB_TILE - 1) / LB_TILE;
+	const auto mx = [](int x, int y) { return y > x ? y : x; };
+	for(int64_t t = blockIdx.x; t < n_tiles; t += gridDim.x)
+	{
+		const int64_t top = ns - 1 - t * LB_TILE;
+		if(top < 0) break;
+		// first head after the tile: warp 0 reads 8 x 32 run heads per step
+		if(threadIdx.x < NH_LANES)
+		{
+			long long found = ns;
+			for(int64_t p = top + 1; p < ns; p += 8 * NH_LANES)
+			{
+				u32 hit = 0;
+				int r0 = 0;
+#pragma unroll
+				for(int r = 7; r >= 0; r--)
+				{
+					const int64_t q = p + r * NH_LANES + threadIdx.x;
+					const bool on = q < ns && seg_head[q];
+#ifndef AGPU_EMU
+					const u32 m = __ballot_sync(0xffffffffu, on);
+#else
+					const u32 m = on ? 1u : 0u;
+#endif
+					if(m) { hit = m; r0 = r; }
+				}
+				if(hit) { found = p + r0 * NH_LANES + __ffs((int)hit) - 1; break; }
+			}
+			if(threadIdx.x == 0) s_after = found;
+		}
+		int h[LB_ROWS];
+#pragma unroll
+		for(int j = 0; j < LB_ROWS; j++)
+		{
+			const int k = j * LB_THREADS + threadIdx.x;
+			h[j] = (top - k >= 0 && seg_head[top - k]) ? k : -1;
+		}
+		lb_rows_scan(h, -1, mx, s_tot);      // its barrier also publishes s_after
+		const long long after = s_after;
+#pragma unroll
+		for(int j = 0; j < LB_ROWS; j++)
+		{
+			const int64_t s = top - (j * LB_THREADS + threadIdx.x);
+			if(s >= 0) nhead[s] = h[j] >= 0 ? top - h[j] : after;
+		}
 		BLOCK_SYNC();
 	}
 }

@@ -147,6 +147,89 @@ DEV int64_t lb_tile_prefix(const lb_ctl &c, int chain, int64_t tile, int64_t agg
 	return (int64_t)s_pre[chain];
 }
 
+// the same for two chains whose aggregates are known together: resolved side by side by two warps, one barrier
+DEV void lb_tile_prefix2(const lb_ctl &c, int chain_a, int chain_b, int64_t tile, int64_t agg_a, int64_t agg_b, int64_t *pre_a, int64_t *pre_b)
+{
+	SHARED long long s_pre2[2];
+#ifndef AGPU_EMU
+	if(blockDim.x >= 64)
+	{
+		const int w = threadIdx.x >> 5;
+		if(w < 2)
+		{
+			const int64_t r = lb_resolve_warp(c, w ? chain_b : chain_a, tile, w ? agg_b : agg_a);
+			if((threadIdx.x & 31) == 0) s_pre2[w] = r;
+		}
+	}
+	else
+#endif
+	if(threadIdx.x == 0) { s_pre2[0] = lb_resolve(c, chain_a, tile, agg_a); s_pre2[1] = lb_resolve(c, chain_b, tile, agg_b); }
+	BLOCK_SYNC();
+	*pre_a = (int64_t)s_pre2[0];
+	*pre_b = (int64_t)s_pre2[1];
+}
+
+// ---- tiles held in registers: thread t owns the elements t, t + LB_THREADS, t + 2 LB_THREADS, ... of the tile (LB_ROWS of them,
+// every global access of a row coalesced).  lb_rows_scan turns them into exclusive prefixes in tile order with warp shuffles;
+// the (row, warp) totals go through shared memory once, so a scan costs one barrier and no bank conflicts.
+#ifndef AGPU_EMU
+#define LB_THREADS 256           // the CTA of LAUNCH_LB
+#else
+#define LB_THREADS 1             // kernel-logic build: one thread per CTA owns the whole tile
+#endif
+#define LB_ROWS (LB_TILE / LB_THREADS)
+#define LB_ROW_TOTALS (LB_ROWS * LB_THREADS / 32 + 1)
+
+// v[j] <- combine of the tile's elements before element j of this thread; returns the combine of the whole tile.  `s_tot`: shared
+// scratch of LB_ROW_TOTALS values, not reused before the next barrier.  The values of one scan are combined in a different order
+// than an element-by-element loop, so `op` must be associative and commutative; int sums wrap (compute them as unsigned).
+template<typename T, typename Op> DEV T lb_rows_scan(T (&v)[LB_ROWS], T ident, Op op, T *s_tot)
+{
+#ifndef AGPU_EMU
+	static_assert(LB_ROWS * LB_THREADS / 32 == 64, "lb_rows_scan: 64 (row, warp) totals");
+	const unsigned FULL = 0xffffffffu;
+	const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+	const int NW = LB_THREADS / 32;
+	T ex[LB_ROWS];
+#pragma unroll
+	for(int j = 0; j < LB_ROWS; j++)
+	{
+		T inc = v[j];
+#pragma unroll
+		for(int o = 1; o < 32; o <<= 1) { const T y = __shfl_up_sync(FULL, inc, o); if(lane >= o) inc = op(y, inc); }
+		const T up = __shfl_up_sync(FULL, inc, 1);
+		ex[j] = lane > 0 ? up : ident;
+		if(lane == 31) s_tot[j * NW + w] = inc;
+	}
+	__syncthreads();
+	// exclusive prefixes of the 64 totals in (row, warp) order, by every warp: lane l holds totals l and 32 + l
+	T a = s_tot[lane], b = s_tot[32 + lane];
+#pragma unroll
+	for(int o = 1; o < 32; o <<= 1)
+	{
+		const T ya = __shfl_up_sync(FULL, a, o), yb = __shfl_up_sync(FULL, b, o);
+		if(lane >= o) { a = op(ya, a); b = op(yb, b); }
+	}
+	const T ta = __shfl_sync(FULL, a, 31), tb = __shfl_sync(FULL, b, 31);
+	T ea = __shfl_up_sync(FULL, a, 1), eb = __shfl_up_sync(FULL, b, 1);
+	if(lane == 0) { ea = ident; eb = ident; }
+	eb = op(ta, eb);
+#pragma unroll
+	for(int j = 0; j < LB_ROWS; j++)
+	{
+		const int e = j * NW + w;                 // j * NW < 32 decides the half at compile time (j is unrolled, w < NW)
+		const T p = j * NW < 32 ? __shfl_sync(FULL, ea, e & 31) : __shfl_sync(FULL, eb, e & 31);
+		v[j] = op(p, ex[j]);
+	}
+	return op(ta, tb);
+#else
+	(void)s_tot;
+	T run = ident;
+	for(int j = 0; j < LB_ROWS; j++) { const T x = v[j]; v[j] = run; run = op(run, x); }
+	return run;
+#endif
+}
+
 // ---- generic scans ---------------------------------------------------------------------------------------------------------
 // exclusive prefix sum of int32 values (mode 0) or of the flags (v[i] >= 0) (mode 1) into int64: out[i], out[n] = total
 KERNEL k_lb_scan_i32(lb_ctl c, const int32_t *v, int64_t n, int mode, int64_t *out)

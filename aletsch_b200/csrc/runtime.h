@@ -328,7 +328,7 @@ inline void lb_destroy(agpu_ctx *ctx)
 #define LAUNCH_LB(ctx, kern, n_tiles, ...) do { int64_t nt_ = (int64_t)(n_tiles); if(nt_ > 0) { unsigned g_ = LB_GRID(ctx, nt_); agpu::lb_ctl lc_; \
 	unsigned ep_; unsigned long long tb_; TRY(lb_prepare(ctx, nt_, g_, &tb_, &ep_)); \
 	lc_.status = (agpu::u64*)(ctx)->lb_status; lc_.ticket = (ctx)->lb_ticket; lc_.stride = (ctx)->lb_stride; lc_.ticket_base = tb_; lc_.epoch = ep_; \
-	prof_begin(ctx, #kern); kern<<<g_, 256, 0, (ctx)->stream>>>(lc_, __VA_ARGS__); prof_end(ctx); (ctx)->launches++; } } while(0)
+	prof_begin(ctx, #kern); kern<<<g_, LB_THREADS, 0, (ctx)->stream>>>(lc_, __VA_ARGS__); prof_end(ctx); (ctx)->launches++; } } while(0)
 #else
 #define LAUNCH_LB(ctx, kern, n_tiles, ...) do { int64_t nt_ = (int64_t)(n_tiles); if(nt_ > 0) { unsigned g_ = 2; agpu::lb_ctl lc_; \
 	unsigned ep_; unsigned long long tb_; TRY(lb_prepare(ctx, nt_, g_, &tb_, &ep_)); \
