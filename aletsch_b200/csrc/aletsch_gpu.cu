@@ -14,6 +14,7 @@
 #include "k_support.h"
 #include "k_unpack.h"
 #include "k_fetch.h"
+#include "k_regroup.h"
 
 #include <algorithm>
 #include <atomic>
@@ -880,5 +881,6 @@ int agpu_batch_graph(agpu_ctx *ctx, agpu_batch *b, const agpu_params *p)
 #include "abi_support.inc"
 #include "abi_preview.inc"
 #include "abi_packed.inc"
+#include "abi_regroup.inc"
 
 }

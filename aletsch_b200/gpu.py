@@ -102,7 +102,8 @@ ABI_SYMBOLS = ["agpu_default_params", "agpu_create", "agpu_destroy", "agpu_last_
                "agpu_profile_read", "agpu_group_resolve", "agpu_debug_sort_perm", "agpu_similarity_batch", "agpu_group_resolve_batch", "agpu_splices_fetch", "agpu_batch_bundle_counts",
                "agpu_batch_group_bridge", "agpu_group_fetch", "agpu_batch_phase_set", "agpu_phase_fetch", "agpu_batch_revise", "agpu_revise_fetch", "agpu_batch_upload_packed", "agpu_reserved", "agpu_reserve", "agpu_blocking_sync", "agpu_upload_async",
                "agpu_batch_results", "agpu_d2h_bytes", "agpu_pinned_match",
-               "agpu_batch_group_support", "agpu_support_fetch", "agpu_batch_coverage_edit", "agpu_batch_preview", "agpu_preview_fetch"]
+               "agpu_batch_group_support", "agpu_support_fetch", "agpu_batch_coverage_edit", "agpu_batch_preview", "agpu_preview_fetch",
+               "agpu_batch_gather"]
 
 
 def load(lib_path=None):
@@ -129,6 +130,7 @@ def load(lib_path=None):
     L.agpu_batch_upload.argtypes = [C.c_void_p, C.POINTER(BatchIn), C.POINTER(C.c_void_p)]
     L.agpu_batch_adopt.argtypes = [C.c_void_p, C.POINTER(BatchIn), C.POINTER(C.c_void_p)]
     L.agpu_batch_upload_packed.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]
+    L.agpu_batch_gather.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]
     L.agpu_batch_free.argtypes = [C.c_void_p, C.c_void_p]
     L.agpu_batch_reset.argtypes = [C.c_void_p, C.c_void_p]
     for n in ("evidence", "graph", "cluster", "bridge", "bridge_all"):
@@ -192,7 +194,14 @@ def _arr(ptr, n, dtype=None):
 
 
 class AgpuError(RuntimeError):
-    pass
+    """a failed ABI call; `rc` is its return code (AGPU_ERR_*)"""
+
+    def __init__(self, msg, rc=None):
+        super().__init__(msg)
+        self.rc = rc
+
+
+AGPU_ERR_ARG, AGPU_ERR_CUDA, AGPU_ERR_OOM, AGPU_ERR_INPUT, AGPU_ERR_CAPACITY = -1, -2, -3, -4, -5
 
 
 class Context:
@@ -216,7 +225,7 @@ class Context:
 
     def check(self, rc, what):
         if rc != 0:
-            raise AgpuError("%s failed with %d: %s" % (what, rc, self.L.agpu_last_error(self.h).decode()))
+            raise AgpuError("%s failed with %d: %s" % (what, rc, self.L.agpu_last_error(self.h).decode()), rc)
 
     def sync(self):
         self.check(self.L.agpu_sync(self.h), "agpu_sync")
@@ -275,6 +284,20 @@ class Context:
 
     def adopt(self, batch_in_device, keepalive=None):
         return Batch(self, batch_in_device, True, keepalive)
+
+    def gather(self, batches, picks):
+        """agpu_batch_gather: a new Batch on this context whose bundle k is bundle picks[k][1] of batches[picks[k][0]], copied on the
+        device.  `batches` may live on other contexts of the same device; they may be freed once this returns."""
+        sel = np.asarray(picks, np.int32).reshape(-1, 2)
+        src = np.ascontiguousarray(sel[:, 0])
+        bun = np.ascontiguousarray(sel[:, 1])
+        if any(getattr(b, "h", None) is None for b in batches):
+            raise ValueError("gather: a source batch has been freed")
+        tab = (C.c_void_p * max(len(batches), 1))(*[b.h.value for b in batches])
+        h = C.c_void_p()
+        self.check(self.L.agpu_batch_gather(self.h, len(batches), tab, len(sel), src.ctypes.data, bun.ctypes.data, C.byref(h)),
+                   "agpu_batch_gather")
+        return Batch.own(self, h, len(sel))
 
     def sort_perm(self, keys):
         keys = np.ascontiguousarray(keys, np.int32)
@@ -380,6 +403,13 @@ class Batch:
         name = "agpu_batch_adopt" if adopt else ("agpu_batch_upload_packed" if hasattr(bin_struct, "hit_meta") else "agpu_batch_upload")
         ctx.check(getattr(ctx.L, name)(ctx.h, C.byref(bin_struct), C.byref(h)), name)
         self.h = h
+
+    @classmethod
+    def own(cls, ctx, handle, n_bundles):
+        """a Batch around a handle an ABI call returned (e.g. agpu_batch_gather); freed with the object"""
+        b = cls.__new__(cls)
+        b.ctx, b.keep, b.nb, b.hit_off, b.h = ctx, None, n_bundles, None, handle
+        return b
 
     def free(self):
         if getattr(self, "h", None) and self.ctx.h:

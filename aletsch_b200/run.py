@@ -5,7 +5,9 @@
 One sample per BAM.  The files are decoded on the host (host/bamio.cc), cut into bundles by the packer (the record loop of
 meta/generator.cc:77-201), and the whole batch goes through bundle::bridge on the device; with --clusters the bundles are also
 clustered across samples (bundle_group::resolve per 1 Mb region and strand) and every cluster is re-bridged against its combined
-splice graph (assembler::bridge).  Prints one summary line per sample and the totals; the results themselves are available
+splice graph (assembler::bridge).  A job larger than one device batch (include/aletsch_gpu.h, BATCHING RULE) is cut by
+position (clusters.device_batches); with --clusters its bundles are then regrouped on the device by cluster (clusters.cluster_pass).
+Prints one summary line per sample and the totals; the results themselves are available
 through the fetch calls of aletsch_b200.gpu.Batch (this tool is a usage example, not a replacement for the assembler).
 """
 import argparse
@@ -15,6 +17,7 @@ import time
 
 import numpy as np
 
+from .clusters import cluster_pass, device_batches
 from . import gpu as G
 from . import hostlib as H
 
@@ -52,9 +55,40 @@ def main(argv=None):
     t1 = time.time()
     gp = G.default_params(library_type=lt, max_group_size=args.max_group_size, min_grouping_similarity=args.min_grouping_similarity)
     ctx = G.Context(args.device)
+    out = {"samples": len(recs), "bundles": batch.n_bundles, "decode_pack_s": round(t1 - t0, 3)}
+    parts = device_batches(batch)
+    if len(parts) > 1:
+        # more than one device batch (include/aletsch_gpu.h, BATCHING RULE): cut by position; with --clusters the bundles are
+        # regrouped on the device by cross-sample cluster (clusters.cluster_pass), else every part runs on its own
+        out["device_batches"] = len(parts)
+        if args.clusters:
+            srcs = [ctx.upload(p.view(), keepalive=p) for p in parts]
+            res = cluster_pass(ctx, parts, srcs, gp)
+            for s in srcs:
+                s.free()
+            out["clusters_of_bundles"] = sum(len(c) for c in res.clusters)
+            bts = res.batches
+        else:
+            def bridged(p):
+                bt = ctx.upload(p.view(), keepalive=p)
+                bt.bridge_all(gp)
+                return bt
+            bts = (bridged(p) for p in parts)
+        tot, phases = {}, 0
+        for bt in bts:
+            bt.graph(gp)
+            phases += int(sum(len(p["phase_cnt"]) for p in bt.phase_set()))
+            for n, v in bt.counts().items():
+                tot[n] = tot.get(n, 0) + v
+            bt.free()
+        out.update(tot)
+        out["distinct_phases"] = phases
+        out["device_s"] = round(time.time() - t1, 3)
+        ctx.close()
+        print(json.dumps(out))
+        return 0
     bt = ctx.upload(batch.view(), keepalive=batch)
     bt.bridge_all(gp)
-    out = {"samples": len(recs), "bundles": batch.n_bundles, "decode_pack_s": round(t1 - t0, 3)}
     if args.clusters and batch.n_bundles:
         off, val = bt.fetch_splices()
         a = batch.a

@@ -202,6 +202,22 @@ int agpu_batch_adopt(agpu_ctx *ctx, const agpu_batch_in *in_device, agpu_batch *
 void agpu_batch_free(agpu_ctx *ctx, agpu_batch *b);
 /* forget all derived state (chains, coverage, fragments, graph ...) but keep the uploaded hits */
 int agpu_batch_reset(agpu_ctx *ctx, agpu_batch *b);
+/* A new batch holding n_sel bundles taken from existing batches: bundle k of *out is bundle sel_bundle[k] of src[sel_src[k]],
+ * copied device to device (aletsch_b200/clusters.py uses it to cut a job a second time, by cross-sample cluster, without sending
+ * the hits over PCIe again).  The output is a fresh batch like the result of agpu_batch_upload: it owns copies of bundle_hit_off,
+ * pos, rpos, mpos, isize, xs, qid, cigar_off and cigar on the device, bundle_tid and bundle_sample on the host, and no derived
+ * state.  strand is always per hit (a source uploaded with bundle_strand only has that strand expanded to its hits); rpos is the
+ * source's device array, uploaded or derived; bundle_sample is kept only if every source has it; flag is not carried (no kernel
+ * reads it).  A bundle may be selected more than once; n_sel == 0 gives a valid empty batch.
+ * Sources may come from any upload entry or agpu_batch_adopt and may belong to other contexts on the same device as ctx: the call
+ * orders itself after the work already queued on each source's context stream (device-side event waits) and ends with a stream
+ * synchronisation, after which the sources may be reset or freed.  No other call may run on a source while the gather runs.
+ * Errors: AGPU_ERR_ARG for an index out of range, a NULL source, a source on another device or a source with coverage edits
+ * (agpu_batch_coverage_edit: per-hit state that is not regrouped); AGPU_ERR_CAPACITY when the output would hold 2^32 or more CIGAR
+ * operations (cigar_off is 32 bits).  Nothing partial is kept on any error.  The packing contract is not checked here: a
+ * violation in a selected bundle surfaces at the output's agpu_batch_evidence, as it would have in the source. */
+int agpu_batch_gather(agpu_ctx *ctx, int32_t n_src, agpu_batch *const *src, int32_t n_sel, const int32_t *sel_src, const int32_t *sel_bundle,
+		agpu_batch **out);
 
 /* ---- stages (asynchronous on the ctx stream unless noted) ----------------------------- */
 int agpu_batch_evidence(agpu_ctx *ctx, agpu_batch *b, const agpu_params *p);
