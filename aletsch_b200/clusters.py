@@ -153,14 +153,23 @@ def cluster_pass(ctx, parts, batches, params, support=False, times=None):
     out.n_clusters = len(cstart) - 1
     span = np.concatenate([bundle_spans(p) for p in parts])[glob]
     hits = np.concatenate([np.diff(p.a["bundle_hit_off"]) for p in parts])[glob]
-    cuts = _cuts(np.add.reduceat(span, cstart[:-1]), np.add.reduceat(hits, cstart[:-1]), unit="cluster")
     part_of = np.searchsorted(base, glob, "right") - 1
     origin = np.stack([part_of, glob - base[part_of], glob], axis=1).astype(np.int64)
-    clock.lap("plan")
-    # 4. per output batch: gather, bundle::bridge, assembler::bridge on its clusters, the support passes
+    run_clusters(ctx, batches, origin[:, :2], span, hits, cstart, params, out, clock, support, origin)
+    return out
+
+
+def run_clusters(ctx, sources, picks, span, hits, cstart, params, out, clock, support, origin):
+    """steps 3 and 4 of the pass on bundles laid out cluster by cluster: bundle k of the layout is bundle picks[k][1] of
+    sources[picks[k][0]], with window estimate span[k] and hits[k]; cluster j is the layout range [cstart[j], cstart[j + 1]).
+    Cuts the layout at cluster boundaries under the batching rule (ValueError for a cluster larger than one device batch), then
+    per output batch: gather, bundle::bridge, assembler::bridge on its clusters, the support passes.  Appends to `out` (a
+    ClusterPass), with origin[k] as the origin row of bundle k."""
+    cuts = _cuts(np.add.reduceat(span, cstart[:-1]), np.add.reduceat(hits, cstart[:-1]), unit="cluster") if len(cstart) > 1 else [0]
+    clock.lap("plan", add=True)
     for k0, k1 in zip(cuts[:-1], cuts[1:]):
         b0, b1 = int(cstart[k0]), int(cstart[k1])
-        bt = ctx.gather(batches, origin[b0:b1, :2])
+        bt = ctx.gather(sources, picks[b0:b1])
         out.batches.append(bt)
         out.origin.append(origin[b0:b1])
         clock.lap("gather", add=True)
@@ -174,7 +183,6 @@ def cluster_pass(ctx, parts, batches, params, support=False, times=None):
         if support:
             out.support.append(_group_support(bt, multi, params) if multi else [])
             clock.lap("group_support", per_batch=True)
-    return out
 
 
 class _Clock:

@@ -25,6 +25,8 @@
 
 #ifdef AGPU_EMU
 thread_local agpu_emu_dim threadIdx, blockIdx, blockDim, gridDim;
+// marks the emulation build for its callers: its "device" pointers (agpu_batch_inputs) are host memory
+extern "C" const int agpu_emu_build = 1;
 #endif
 
 using namespace agpu;

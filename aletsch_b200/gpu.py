@@ -103,7 +103,7 @@ ABI_SYMBOLS = ["agpu_default_params", "agpu_create", "agpu_destroy", "agpu_last_
                "agpu_batch_group_bridge", "agpu_group_fetch", "agpu_batch_phase_set", "agpu_phase_fetch", "agpu_batch_revise", "agpu_revise_fetch", "agpu_batch_upload_packed", "agpu_reserved", "agpu_reserve", "agpu_blocking_sync", "agpu_upload_async",
                "agpu_batch_results", "agpu_d2h_bytes", "agpu_pinned_match",
                "agpu_batch_group_support", "agpu_support_fetch", "agpu_batch_coverage_edit", "agpu_batch_preview", "agpu_preview_fetch",
-               "agpu_batch_gather"]
+               "agpu_batch_gather", "agpu_batch_inputs"]
 
 
 def load(lib_path=None):
@@ -131,6 +131,7 @@ def load(lib_path=None):
     L.agpu_batch_adopt.argtypes = [C.c_void_p, C.POINTER(BatchIn), C.POINTER(C.c_void_p)]
     L.agpu_batch_upload_packed.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]
     L.agpu_batch_gather.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(C.c_void_p)]
+    L.agpu_batch_inputs.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(BatchIn)]
     L.agpu_batch_free.argtypes = [C.c_void_p, C.c_void_p]
     L.agpu_batch_reset.argtypes = [C.c_void_p, C.c_void_p]
     for n in ("evidence", "graph", "cluster", "bridge", "bridge_all"):
@@ -168,6 +169,7 @@ def load(lib_path=None):
     L.agpu_profile_enable.argtypes = [C.c_void_p, C.c_int]
     L.agpu_profile_reset.argtypes = [C.c_void_p]
     L.agpu_profile_read.argtypes = [C.c_void_p, C.c_char_p, C.c_size_t]
+    L.host_memory = hasattr(L, "agpu_emu_build")      # the kernel-logic emulation build (tests/emu): its "device" arrays are host memory
     return L
 
 
@@ -389,6 +391,14 @@ def reorder_lists(off, val, order):
     if got != total:
         raise ValueError("reorder_lists: index outside the lists")
     return noff, nval[:total]
+
+
+class _DeviceArray:
+    """__cuda_array_interface__ of one device column of a batch; holds the batch so that it is not collected under the tensor"""
+
+    def __init__(self, ptr, n, typestr, owner):
+        self.owner = owner
+        self.__cuda_array_interface__ = {"shape": (n,), "typestr": typestr, "data": (ptr, False), "version": 3, "strides": None}
 
 
 class Batch:
@@ -642,6 +652,32 @@ class Batch:
             d.update(fcs[k])
             out.append(d)
             m0 += n
+        return out
+
+    INPUT_COLUMNS = [("bundle_hit_off", "nb1", "<i8"), ("pos", "nh", "<i4"), ("rpos", "nh", "<i4"), ("mpos", "nh", "<i4"),
+                     ("isize", "nh", "<i4"), ("strand", "nh", "|i1"), ("bundle_strand", "nb", "|i1"), ("xs", "nh", "|i1"),
+                     ("qid", "nh", "<i8"), ("cigar_off", "nh1", "<i4"), ("cigar", "nc", "<i4")]
+
+    def input_columns(self):
+        """agpu_batch_inputs: the input columns the stages read, as zero-copy torch tensors over the batch's device arrays (CPU
+        tensors over host memory on the emulation build), unsigned columns viewed as signed ones of the same width.  Of strand and
+        bundle_strand only the one the batch has is present.  Valid until the batch is freed; no stage writes them."""
+        import torch
+        v = BatchIn()
+        self.ctx.check(self.ctx.L.agpu_batch_inputs(self.ctx.h, self.h, C.byref(v)), "agpu_batch_inputs")
+        size = {"nb": v.n_bundles, "nb1": v.n_bundles + 1, "nh": v.n_hits, "nh1": v.n_hits + 1, "nc": v.n_cigar}
+        out = {}
+        for name, n, typestr in self.INPUT_COLUMNS:
+            ptr, n = getattr(v, name), int(size[n])
+            if not ptr:
+                continue
+            dt = np.dtype(typestr)
+            if n == 0:
+                out[name] = torch.empty(0, dtype=torch.from_numpy(np.zeros(0, dt)).dtype)
+            elif self.ctx.L.host_memory:
+                out[name] = torch.from_numpy(np.ctypeslib.as_array(C.cast(ptr, C.POINTER(np.ctypeslib.as_ctypes_type(dt))), shape=(n,)))
+            else:
+                out[name] = torch.as_tensor(_DeviceArray(ptr, n, typestr, self), device="cuda")
         return out
 
     def bundle_counts(self):

@@ -9,9 +9,16 @@ splice graph (assembler::bridge).  A job larger than one device batch (include/a
 position (clusters.device_batches); with --clusters its bundles are then regrouped on the device by cluster (clusters.cluster_pass).
 Prints one summary line per sample and the totals; the results themselves are available
 through the fetch calls of aletsch_b200.gpu.Batch (this tool is a usage example, not a replacement for the assembler).
+
+Under torchrun (WORLD_SIZE > 1, one process per GPU, NCCL) the samples are sharded: rank r decodes the files with index
+i % world == r, and with --clusters every cluster's bundles are moved to one GPU for the cluster pass
+(shard.cluster_pass_sharded); rank 0 prints the totals over all ranks.
+
+    torchrun --nproc-per-node 2 -m aletsch_b200.run --clusters a.bam b.bam c.bam
 """
 import argparse
 import json
+import os
 import sys
 import time
 
@@ -38,6 +45,8 @@ def main(argv=None):
                          "which drops every region's first hit and the last region of the last chromosome")
     args = ap.parse_args(argv)
     lt = {"unstranded": H.UNSTRANDED, "first": H.FR_FIRST, "second": H.FR_SECOND, "auto": None}[args.library_type]
+    if int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        return _sharded(args, lt)
     t0 = time.time()
     recs, chrom_len = [], None
     for path in args.bams:
@@ -127,6 +136,85 @@ def main(argv=None):
     bt.free()
     ctx.close()
     print(json.dumps(out))
+    return 0
+
+
+def _sharded(args, lt):
+    """the run with one process per GPU: samples dealt to ranks by file index, the cluster pass over all of them"""
+    import torch
+    import torch.distributed as dist
+    from .shard import bundle_keys, cluster_pass_sharded
+    local = int(os.environ.get("LOCAL_RANK", "0"))
+    torch.cuda.set_device(local)
+    dist.init_process_group("nccl", device_id=torch.device("cuda", local))
+    try:
+        rank, world = dist.get_rank(), dist.get_world_size()
+        t0 = time.time()
+        mine = [i for i in range(len(args.bams)) if i % world == rank]
+        recs, chrom_len = [], None
+        for i in mine:
+            r, cl = H.read_bam(args.bams[i])
+            if chrom_len is not None and not np.array_equal(cl, chrom_len):
+                raise SystemExit("%s: reference dictionary differs from the first file's" % args.bams[i])
+            chrom_len = cl
+            recs.append(r)
+            print("rank %d: %s: %d records" % (rank, args.bams[i], r["n"]), file=sys.stderr)
+        dicts = [None] * world
+        dist.all_gather_object(dicts, None if chrom_len is None else [int(x) for x in chrom_len])
+        ref = dicts[0]                   # rank 0 holds file 0
+        for r, d in enumerate(dicts):
+            if d is not None and d != ref:      # file r is the first file of rank r
+                raise SystemExit("%s: reference dictionary differs from the first file's" % args.bams[r])
+        if lt is None:
+            got = [None]
+            if rank == 0:
+                pv = H.infer_library_type(recs[0], H.default_packer_params(H.UNSTRANDED))
+                got[0] = pv["library_type"]
+                print("inferred library type %d from %s: %s" % (got[0], args.bams[0], pv), file=sys.stderr)
+            dist.broadcast_object_list(got, src=0)
+            lt = got[0]
+        batch = H.pack(recs, H.default_packer_params(lt), sample_ids=mine, chrom_len=None if args.whole_file else np.array(ref, np.int32),
+                       region_length=REGION)
+        t1 = time.time()
+        gp = G.default_params(library_type=lt, max_group_size=args.max_group_size, min_grouping_similarity=args.min_grouping_similarity)
+        ctx = G.Context(local)
+        parts = device_batches(batch) if batch.n_bundles else []
+        out = {"bundles": batch.n_bundles, "device_batches": len(parts), "clusters_of_bundles": 0}
+        if args.clusters:
+            srcs = [ctx.upload(p.view(), keepalive=p) for p in parts]
+            res = cluster_pass_sharded(ctx, parts, srcs, bundle_keys(batch), gp)
+            for s in srcs:
+                s.free()
+            out["clusters_of_bundles"] = sum(len(c) for c in res.clusters)
+            bts = res.batches
+        else:
+            def bridged(p):
+                bt = ctx.upload(p.view(), keepalive=p)
+                bt.bridge_all(gp)
+                return bt
+            bts = (bridged(p) for p in parts)
+        phases = 0
+        for bt in bts:
+            bt.graph(gp)
+            phases += int(sum(len(p["phase_cnt"]) for p in bt.phase_set()))
+            for n, v in bt.counts().items():
+                out[n] = out.get(n, 0) + v
+            bt.free()
+        out["distinct_phases"] = phases
+        out["decode_pack_s"], out["device_s"] = t1 - t0, time.time() - t1
+        ctx.close()
+        every = [None] * world
+        dist.all_gather_object(every, out)
+        if rank == 0:
+            tot = {"samples": len(args.bams)}
+            for o in every:
+                for n, v in o.items():
+                    tot[n] = max(tot.get(n, 0), v) if n.endswith("_s") else tot.get(n, 0) + v
+            tot["decode_pack_s"], tot["device_s"] = round(tot["decode_pack_s"], 3), round(tot["device_s"], 3)
+            tot["ranks"] = world
+            print(json.dumps(tot))
+    finally:
+        dist.destroy_process_group()
     return 0
 
 

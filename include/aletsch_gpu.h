@@ -218,6 +218,14 @@ int agpu_batch_reset(agpu_ctx *ctx, agpu_batch *b);
  * violation in a selected bundle surfaces at the output's agpu_batch_evidence, as it would have in the source. */
 int agpu_batch_gather(agpu_ctx *ctx, int32_t n_src, agpu_batch *const *src, int32_t n_sel, const int32_t *sel_src, const int32_t *sel_bundle,
 		agpu_batch **out);
+/* The input columns the stages read, as DEVICE pointers, with the batch's counts: bundle_hit_off, pos, rpos, mpos, isize, strand
+ * (per hit) or bundle_strand (per bundle; the other one is NULL), xs, qid, cigar_off and cigar.  bundle_tid, bundle_sample and
+ * flag are returned as NULL: the first two live on the host side of the batch, flag is never uploaded.  rpos is the uploaded or
+ * the derived array.  A batch built by agpu_batch_gather always has rpos and a per-hit strand.  No stage writes these arrays, so
+ * the pointers stay valid and unchanged until agpu_batch_free, e.g. as send buffers of a transfer between GPUs
+ * (aletsch_b200/shard.py), while stages run on the batch.  Builds without a device (the kernel-logic emulation) return host
+ * pointers.  AGPU_ERR_ARG for NULL arguments. */
+int agpu_batch_inputs(agpu_ctx *ctx, agpu_batch *b, agpu_batch_in *out);
 
 /* ---- stages (asynchronous on the ctx stream unless noted) ----------------------------- */
 int agpu_batch_evidence(agpu_ctx *ctx, agpu_batch *b, const agpu_params *p);
