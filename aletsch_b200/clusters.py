@@ -9,7 +9,7 @@ holds bundles of all samples at one locus.  So the job is cut twice, in the orde
 
   1. by position (device_batches): evidence on every source batch, then every bundle's splice list (agpu_splices_fetch) -- all
      stage 5 needs;
-  2. stage 5 over the region groups of the whole job, as run.py forms them;
+  2. stage 5 over the region groups of the whole job (chromosome, 1 Mb region, strand: shard.bundle_region_keys);
   3. by cluster: every bundle of the job goes to exactly one output batch, laid out cluster by cluster (members in gv order), cut
      only at cluster boundaries under the same rule; the output batches are built on the device from the bundles already in HBM
      (agpu_batch_gather), then bridged per bundle, re-bridged per cluster and, if asked, given the support passes.
@@ -23,7 +23,7 @@ import time
 import numpy as np
 
 from . import gpu as G
-from .shard import bundle_region_keys
+from .shard import _cluster_pass
 
 MAX_BATCH_SPAN = 3_000_000_000     # window positions per device batch: the coverage index is 32-bit (AGPU_ERR_CAPACITY above 2^32)
 MAX_BATCH_HITS = 60_000_000
@@ -82,11 +82,11 @@ class ClusterPass:
       clusters[i]  its clusters of >= 2 bundles as lists of batch-local bundle indices in gv order (what group_bridge ran on)
       origin[i]    int64 [NB, 3]: per local bundle, the source part, the bundle index in that part and the bundle index in the job
       support[i]   the support rows of its clusters (gpu.Batch.group_support's dicts), when asked for; else None
-    and n_clusters, the stage-5 cluster count of the job, singletons included."""
+    and n_groups / n_clusters, the region-group and stage-5 cluster counts of the job, singletons included."""
 
     def __init__(self):
         self.batches, self.clusters, self.origin, self.support = [], [], [], None
-        self.n_clusters = 0
+        self.n_groups = self.n_clusters = 0
 
     def free(self):
         for b in self.batches:
@@ -111,51 +111,15 @@ def cluster_pass(ctx, parts, batches, params, support=False, times=None):
     parts:   the host sub-batches (hostlib.PackedBatch): contiguous slices, in order, of one job, as device_batches returns them
     batches: the matching device batches (gpu.Batch, on any context of ctx's device), fresh: just uploaded or reset
     params:  gpu.Params, including max_group_size / min_grouping_similarity of stage 5
-    times:   optional dict; receives host-clock seconds of every phase around synchronised work ('evidence', 'stage5', 'plan',
-             'gather', and per output batch lists 'bridge_all', 'group_bridge', 'group_support')
-    The output batches live on ctx.  The caller owns the sources and may free them once this returns."""
-    if len(parts) != len(batches):
-        raise ValueError("cluster_pass: %d host parts but %d device batches" % (len(parts), len(batches)))
-    clock = _Clock(ctx, batches, times)
-    out = ClusterPass()
-    if support:
-        out.support = []
-    base = np.concatenate([[0], np.cumsum([p.n_bundles for p in parts])]).astype(np.int64)
-    n = int(base[-1])
-    # 1. evidence on the sources, then bundle::splices of every bundle of the job
-    offs, vals, vb = [np.zeros(1, np.int64)], [], 0
-    for bt in batches:
-        bt.evidence(params)
-        o, v = bt.fetch_splices()
-        offs.append(o[1:] + vb)
-        vals.append(v)
-        vb += int(o[-1])
-    off = np.concatenate(offs)
-    val = np.concatenate(vals) if vals else np.zeros(0, np.int32)
-    clock.lap("evidence")
-    if n == 0:
-        return out
-    # 2. stage 5 over the region groups (chromosome, 1 Mb region, strand), members in (sample, job index) order, as run.py forms them
-    key = np.concatenate([bundle_region_keys(p) for p in parts])
-    sample = np.concatenate([p.a["bundle_sample"] for p in parts])
-    order = np.lexsort((np.arange(n), sample, key))
-    goff = np.concatenate([[0], np.nonzero(np.diff(key[order]))[0] + 1, [n]]).astype(np.int32)
-    loff, lval = G.reorder_lists(off, val, order)
-    cl_of, _ = G.group_resolve_arrays(ctx, goff, loff, lval, params)
-    cl_of = cl_of[:n]
-    clock.lap("stage5")
-    # 3. layout cluster by cluster (groups in order, clusters in gvv order, members in gv order), cut at cluster boundaries
-    gid = np.repeat(np.arange(len(goff) - 1), np.diff(goff))
-    lay = np.lexsort((np.arange(n), cl_of, gid))
-    glob = order[lay]
-    new = (np.diff(gid[lay]) != 0) | (np.diff(cl_of[lay]) != 0)
-    cstart = np.concatenate([[0], np.nonzero(new)[0] + 1, [n]]).astype(np.int64)
-    out.n_clusters = len(cstart) - 1
-    span = np.concatenate([bundle_spans(p) for p in parts])[glob]
-    hits = np.concatenate([np.diff(p.a["bundle_hit_off"]) for p in parts])[glob]
-    part_of = np.searchsorted(base, glob, "right") - 1
-    origin = np.stack([part_of, glob - base[part_of], glob], axis=1).astype(np.int64)
-    run_clusters(ctx, batches, origin[:, :2], span, hits, cstart, params, out, clock, support, origin)
+    times:   optional dict; receives host-clock seconds of every phase around synchronised work ('evidence', 'signatures', 'stage5',
+             'plan', 'exchange', 'gather', and per output batch lists 'bridge_all', 'group_bridge', 'group_support')
+    The output batches live on ctx.  The caller owns the sources and may free them once this returns.  This is the sharded pass
+    of one rank (shard.cluster_pass_sharded) with keys sample << 32 | job index, so nothing is communicated even when a process
+    group exists."""
+    sample = np.concatenate([p.a["bundle_sample"] for p in parts]).astype(np.int64) if parts else np.zeros(0, np.int64)
+    keys = (sample << 32) | np.arange(len(sample), dtype=np.int64)
+    out = _cluster_pass(ctx, parts, batches, keys, params, support, times, 0, 1)
+    out.origin = [np.stack([o[:, 2], o[:, 3], o[:, 1] & 0xffffffff], axis=1) for o in out.origin]
     return out
 
 

@@ -11,7 +11,8 @@ cluster_pass_sharded builds the rest of the cross-sample pass on that: the same 
 operations and window estimate, every rank computes the same plan (plan_clusters: which rank owns which cluster, single-bundle
 clusters staying where they were ingested), the bundles of every cluster move to its owner (one device gather per peer, the
 batch's device columns sent with NCCL point-to-point, adopted on the receiving side without a copy), and the owner runs
-assembler::bridge and the support passes on its clusters (clusters.run_clusters).
+assembler::bridge and the support passes on its clusters (clusters.run_clusters).  With one rank the same pass runs without any
+communication: that is clusters.cluster_pass.
 Backend: NCCL over NVLink on GPUs; the CPU tests run the same code over gloo.
 """
 import numpy as np
@@ -33,66 +34,8 @@ def assign_units(weights, world, load=None):
     return rank_of
 
 
-def my_units(weights, world, rank):
-    return np.nonzero(assign_units(weights, world) == rank)[0]
-
-
 def _device():
     return torch.device("cuda", torch.cuda.current_device()) if dist.get_backend() == "nccl" else torch.device("cpu")
-
-
-def gather_signatures(lists, keys=None):
-    """all-gather of variable-length sorted int32 lists.
-
-    lists: this rank's splice lists (one per local bundle); keys: optional int64 per list (e.g.
-    sample << 32 | bundle index) carried along.  Returns (all_lists, owner_rank, all_keys) in rank order, the
-    same on every rank.  Two collectives: the per-rank (n_lists, n_values) header, then one padded payload
-    [lengths | keys | values] -- signatures are KBs per bundle, latency not bandwidth matters (SURVEY section 5).
-    """
-    world = dist.get_world_size()
-    dev = _device()
-    n = len(lists)
-    lens = np.array([len(x) for x in lists], np.int64)
-    vals = np.concatenate([np.asarray(x, np.int64) for x in lists]) if n and lens.sum() else np.zeros(0, np.int64)
-    k = np.asarray(keys, np.int64) if keys is not None else np.zeros(n, np.int64)
-    head = torch.tensor([n, int(lens.sum())], dtype=torch.int64, device=dev)
-    heads = [torch.zeros(2, dtype=torch.int64, device=dev) for _ in range(world)]
-    dist.all_gather(heads, head)
-    heads = [h.cpu().numpy() for h in heads]
-    cap = max(int(2 * h[0] + h[1]) for h in heads)
-    mine = torch.zeros(max(cap, 1), dtype=torch.int64, device=dev)
-    payload = np.concatenate([lens, k, vals])
-    if len(payload):
-        mine[:len(payload)] = torch.from_numpy(payload).to(dev)
-    parts = [torch.zeros_like(mine) for _ in range(world)]
-    dist.all_gather(parts, mine)
-    all_lists, owner, all_keys = [], [], []
-    for r in range(world):
-        nr, nv = int(heads[r][0]), int(heads[r][1])
-        p = parts[r].cpu().numpy()
-        ln, kk, vv = p[:nr], p[nr:2 * nr], p[2 * nr:2 * nr + nv]
-        off = np.concatenate([[0], np.cumsum(ln)])
-        for i in range(nr):
-            all_lists.append(vv[off[i]:off[i + 1]].astype(np.int32))
-            owner.append(r)
-            all_keys.append(int(kk[i]))
-    return all_lists, np.array(owner, np.int32), np.array(all_keys, np.int64)
-
-
-def resolve_groups(ctx, lists, params, keys=None):
-    """bundle_group::resolve over the bundles of ALL ranks: gather the signatures, sort them into the canonical
-    (key) order so that every rank sees the same gset order (SURVEY section 4: gset order must be fixed), and run
-    agpu_group_resolve on this rank's GPU.  Returns (groups as lists of (owner_rank, key)), identical on every rank."""
-    from . import gpu as G
-    if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-        all_lists, owner, all_keys = gather_signatures(lists, keys)
-    else:
-        all_lists = [np.asarray(x, np.int32) for x in lists]
-        owner = np.zeros(len(lists), np.int32)
-        all_keys = np.asarray(keys, np.int64) if keys is not None else np.arange(len(lists), dtype=np.int64)
-    order = sorted(range(len(all_lists)), key=lambda i: (int(all_keys[i]), int(owner[i]), i))
-    groups = G.group_resolve(ctx, [all_lists[i] for i in order], params)
-    return [[(int(owner[order[i]]), int(all_keys[order[i]])) for i in g] for g in groups]
 
 
 REGION = 1_000_000      # region_partition_length (util/parameters.cc:42)
@@ -212,8 +155,7 @@ def plan_clusters(keys, region, cluster, owner, hits, span, world):
     keys, region, cluster = np.asarray(keys, np.int64), np.asarray(region, np.int64), np.asarray(cluster, np.int64)
     owner, hits, span = np.asarray(owner, np.int64), np.asarray(hits, np.int64), np.asarray(span, np.int64)
     n = len(keys)
-    order = np.lexsort((keys, region))
-    lay = order[np.lexsort((np.arange(n), cluster[order], region[order]))]
+    lay = np.lexsort((keys, cluster, region))
     new = (np.diff(region[lay]) != 0) | (np.diff(cluster[lay]) != 0)
     cstart = np.concatenate([[0], np.nonzero(new)[0] + 1, [n]]).astype(np.int64) if n else np.zeros(1, np.int64)
     size = np.diff(cstart)
@@ -323,18 +265,23 @@ def cluster_pass_sharded(ctx, parts, batches, keys, params, support=False, times
     and 4 of cluster_pass (clusters.run_clusters) run on this rank's clusters.
 
     Returns a clusters.ClusterPass for this rank's clusters; its origin rows are (ingesting rank, global key, local part, index in
-    the part), the last two -1 for a bundle received from another rank, and n_clusters counts the clusters of the whole job.
-    `.exchange` holds the bundles, hits and bytes this rank sent and received, and the bytes per peer (bytes_to, bytes_from).
-    times: cluster_pass's phases plus 'signatures' (the all-gather), 'plan' and 'exchange'.  Without a process group, or with one rank, the result equals cluster_pass's."""
+    the part), the last two -1 for a bundle received from another rank, and n_groups / n_clusters count the region groups and
+    clusters of the whole job.  `.exchange` holds the bundles, hits and bytes this rank sent and received, and the bytes per peer
+    (bytes_to, bytes_from).  times: cluster_pass's phases.  Without a process group the result equals cluster_pass's."""
+    grouped = dist.is_available() and dist.is_initialized()
+    rank, world = (dist.get_rank(), dist.get_world_size()) if grouped else (0, 1)
+    return _cluster_pass(ctx, parts, batches, keys, params, support, times, rank, world)
+
+
+def _cluster_pass(ctx, parts, batches, keys, params, support, times, rank, world):
+    """the cross-sample cluster pass as rank `rank` of `world`; with world 1 nothing is communicated, whatever process group exists"""
     from .clusters import ClusterPass, _Clock, bundle_spans, run_clusters
     if len(parts) != len(batches):
-        raise ValueError("cluster_pass_sharded: %d host parts but %d device batches" % (len(parts), len(batches)))
+        raise ValueError("cluster pass: %d host parts but %d device batches" % (len(parts), len(batches)))
     keys = np.asarray(keys, np.int64)
     base = np.concatenate([[0], np.cumsum([p.n_bundles for p in parts])]).astype(np.int64)
     if len(keys) != base[-1]:
-        raise ValueError("cluster_pass_sharded: %d keys for %d bundles" % (len(keys), base[-1]))
-    grouped = dist.is_available() and dist.is_initialized()
-    rank, world = (dist.get_rank(), dist.get_world_size()) if grouped else (0, 1)
+        raise ValueError("cluster pass: %d keys for %d bundles" % (len(keys), base[-1]))
     clock = _Clock(ctx, batches, times)
     out = ClusterPass()
     out.support = [] if support else None
@@ -348,6 +295,7 @@ def cluster_pass_sharded(ctx, parts, batches, keys, params, support=False, times
         offs.append(o[1:] + vb)
         vals.append(v)
         vb += int(o[-1])
+    off, val = np.concatenate(offs), np.concatenate(vals) if vals else np.zeros(0, np.int32)
     clock.lap("evidence")
     # 2. one all-gather: signatures with (region key, hits, CIGAR operations, window estimate) per bundle; stage 5 on every rank
     cols = np.zeros((len(keys), 4), np.int64)
@@ -355,10 +303,12 @@ def cluster_pass_sharded(ctx, parts, batches, keys, params, support=False, times
         hit_off = [p.a["bundle_hit_off"] for p in parts]
         cols[:, 0] = np.concatenate([bundle_region_keys(p) for p in parts])
         cols[:, 1] = np.concatenate([np.diff(h) for h in hit_off])
-        cols[:, 2] = np.concatenate([np.diff(p.a["cigar_off"].astype(np.int64)[h]) for p, h in zip(parts, hit_off)])
+        cols[:, 2] = np.concatenate([np.diff(p.a["cigar_off"][h].astype(np.int64)) for p, h in zip(parts, hit_off)])
         cols[:, 3] = np.concatenate([bundle_spans(p) for p in parts])
-    off_all, val_all, keys_all, x, owner, _ = gather_packed(np.concatenate(offs), np.concatenate(vals) if vals else np.zeros(0, np.int32),
-                                                            keys, cols)
+    if world > 1:
+        off_all, val_all, keys_all, x, owner, _ = gather_packed(off, val, keys, cols)
+    else:
+        off_all, val_all, keys_all, x, owner = off, val, keys, cols, np.zeros(len(keys), np.int32)
     clock.lap("signatures")
     n = len(keys_all)
     if n == 0:
@@ -366,6 +316,7 @@ def cluster_pass_sharded(ctx, parts, batches, keys, params, support=False, times
     order, cl_sorted = _resolve_sorted(ctx, off_all, val_all, keys_all, x[:, 0], params)
     cl_of = np.empty(n, np.int64)
     cl_of[order] = cl_sorted
+    out.n_groups = 1 + int(np.count_nonzero(np.diff(x[order, 0])))
     clock.lap("stage5")
     # 3. the plan, the same on every rank
     plan = plan_clusters(keys_all, x[:, 0], cl_of, owner, x[:, 1], x[:, 3], world)

@@ -52,10 +52,13 @@ def _worker(rank, world, port, emu, q):
     batch, lt = _batch()
     gp, _ = parity.params_pair(lt, max_group_size=3)
     sizes = np.diff(batch.a["bundle_hit_off"])
-    mine = shard.my_units(sizes, world, rank)
+    mine = np.nonzero(shard.assign_units(sizes, world) == rank)[0]
     ctx = G.Context(0, lib_path=emu)
     lists, segs, hits = _splice_lists(ctx, batch, gp, mine)
-    groups = shard.resolve_groups(ctx, lists, gp, keys=mine)
+    # one region group of all bundles, keyed by their global indices: clusters in gvv order, members in key order
+    off = np.concatenate([[0], np.cumsum([len(x) for x in lists])])
+    keys, _, cl_of, owner, _ = shard.resolve_region_groups(ctx, off, np.concatenate(lists), mine, np.zeros(len(mine), np.int64), gp)
+    groups = [[(int(owner[i]), int(keys[i])) for i in np.nonzero(cl_of == c)[0]] for c in range(int(cl_of.max()) + 1)]
     ctx.close()
     q.put((rank, mine.tolist(), [x.tolist() for x in lists], [x.tolist() for x in segs], int(hits), groups))
     dist.barrier()
@@ -76,7 +79,7 @@ def test_lpt_assignment_is_balanced_and_total():
     assert list(shard.assign_units([5, 5, 5], 2)) == [0, 1, 0]
 
 
-def test_two_ranks_match_single_process(emu_lib):
+def test_two_ranks_resolve_region_groups_match_single_process(emu_lib):
     world = 2
     port = _free_port()
     ctxm = mp.get_context("spawn")
