@@ -82,10 +82,11 @@ class ClusterPass:
       clusters[i]  its clusters of >= 2 bundles as lists of batch-local bundle indices in gv order (what group_bridge ran on)
       origin[i]    int64 [NB, 3]: per local bundle, the source part, the bundle index in that part and the bundle index in the job
       support[i]   the support rows of its clusters (gpu.Batch.group_support's dicts), when asked for; else None
+      phases[i]    the combined phase set px of each of its clusters (gpu.Batch.group_phase_set's dicts), when asked for; else None
     and n_groups / n_clusters, the region-group and stage-5 cluster counts of the job, singletons included."""
 
     def __init__(self):
-        self.batches, self.clusters, self.origin, self.support = [], [], [], None
+        self.batches, self.clusters, self.origin, self.support, self.phases = [], [], [], None, None
         self.n_groups = self.n_clusters = 0
 
     def free(self):
@@ -105,30 +106,33 @@ def _group_support(bt, clusters, params):
     return _group_support(bt, clusters[:h], params) + _group_support(bt, clusters[h:], params)
 
 
-def cluster_pass(ctx, parts, batches, params, support=False, times=None):
-    """Stage 5, assembler::bridge and (support=True) the support passes over a job cut into several device batches.
+def cluster_pass(ctx, parts, batches, params, support=False, times=None, phases=False):
+    """Stage 5, assembler::bridge, (support=True) the support passes and (phases=True) the clusters' combined phase sets over a
+    job cut into several device batches.
 
     parts:   the host sub-batches (hostlib.PackedBatch): contiguous slices, in order, of one job, as device_batches returns them
     batches: the matching device batches (gpu.Batch, on any context of ctx's device), fresh: just uploaded or reset
     params:  gpu.Params, including max_group_size / min_grouping_similarity of stage 5
     times:   optional dict; receives host-clock seconds of every phase around synchronised work ('evidence', 'signatures', 'stage5',
-             'plan', 'exchange', 'gather', and per output batch lists 'bridge_all', 'group_bridge', 'group_support')
+             'plan', 'exchange', 'gather', and per output batch lists 'bridge_all', 'group_bridge', 'group_support', 'phase_set')
     The output batches live on ctx.  The caller owns the sources and may free them once this returns.  This is the sharded pass
     of one rank (shard.cluster_pass_sharded) with keys sample << 32 | job index, so nothing is communicated even when a process
     group exists."""
     sample = np.concatenate([p.a["bundle_sample"] for p in parts]).astype(np.int64) if parts else np.zeros(0, np.int64)
     keys = (sample << 32) | np.arange(len(sample), dtype=np.int64)
-    out = _cluster_pass(ctx, parts, batches, keys, params, support, times, 0, 1)
+    out = _cluster_pass(ctx, parts, batches, keys, params, support, times, 0, 1, phases)
     out.origin = [np.stack([o[:, 2], o[:, 3], o[:, 1] & 0xffffffff], axis=1) for o in out.origin]
     return out
 
 
-def run_clusters(ctx, sources, picks, span, hits, cstart, params, out, clock, support, origin):
+def run_clusters(ctx, sources, picks, span, hits, cstart, params, out, clock, support, origin, phases=False):
     """steps 3 and 4 of the pass on bundles laid out cluster by cluster: bundle k of the layout is bundle picks[k][1] of
     sources[picks[k][0]], with window estimate span[k] and hits[k]; cluster j is the layout range [cstart[j], cstart[j + 1]).
     Cuts the layout at cluster boundaries under the batching rule (ValueError for a cluster larger than one device batch), then
-    per output batch: gather, bundle::bridge, assembler::bridge on its clusters, the support passes.  Appends to `out` (a
-    ClusterPass), with origin[k] as the origin row of bundle k."""
+    per output batch: gather, bundle::bridge, assembler::bridge on its clusters, the support passes, and the members' phase sets
+    against graphs rebuilt from the updated evidence with every cluster's combined phase set (a cluster lives in one output
+    batch, so this needs nothing from other batches or ranks).  Appends to `out` (a ClusterPass), with origin[k] as the origin
+    row of bundle k."""
     cuts = _cuts(np.add.reduceat(span, cstart[:-1]), np.add.reduceat(hits, cstart[:-1]), unit="cluster") if len(cstart) > 1 else [0]
     clock.lap("plan", add=True)
     for k0, k1 in zip(cuts[:-1], cuts[1:]):
@@ -147,6 +151,12 @@ def run_clusters(ctx, sources, picks, span, hits, cstart, params, out, clock, su
         if support:
             out.support.append(_group_support(bt, multi, params) if multi else [])
             clock.lap("group_support", per_batch=True)
+        if phases:
+            if multi:
+                bt.graph(params)
+                bt._run("phase_set")
+            out.phases.append(bt.group_phase_set(multi) if multi else [])
+            clock.lap("phase_set", per_batch=True)
 
 
 class _Clock:

@@ -158,6 +158,13 @@ struct batch_derived
 	int64_t n_phase = 0, n_phase_val = 0;
 	dbuf<int32_t> ph_val, ph_len, ph_cnt;
 	dbuf<int64_t> ph_off, ph_boff;
+	// combined phase sets of bundle clusters (agpu_batch_group_phase_set): distinct lists per cluster in element order, their
+	// coordinates in ph_val
+	bool gphase_built = false;
+	int32_t gph_ng = 0;
+	int64_t n_gphase = 0;
+	dbuf<int32_t> gph_len, gph_cnt;
+	dbuf<int64_t> gph_off, gph_boff;
 
 	// boundary revision (identify_boundaries / remove_false_boundaries): added edges and vertex annotations, in the vertex
 	// layout of the graphs
@@ -240,6 +247,14 @@ static int check_err(agpu_ctx *ctx, agpu_batch *b, const char *stage)
 		return (k == ERR_CAP) ? AGPU_ERR_CAPACITY : AGPU_ERR_INPUT;
 	}
 	return AGPU_OK;
+}
+
+// the combined phase sets refer to the members' coordinates: they go whenever those do (agpu_batch_phase_set), and with a new
+// group pass (agpu_batch_group_bridge)
+static void drop_group_phase_set(agpu_batch *b)
+{
+	b->gph_off.release(); b->gph_len.release(); b->gph_cnt.release(); b->gph_boff.release();
+	b->gphase_built = false; b->gph_ng = 0; b->n_gphase = 0;
 }
 
 // device-wide exclusive prefix sums, one launch each (lookback.h): out[i] = sum of v[0..i), out[n] = total

@@ -103,7 +103,7 @@ ABI_SYMBOLS = ["agpu_default_params", "agpu_create", "agpu_destroy", "agpu_last_
                "agpu_batch_group_bridge", "agpu_group_fetch", "agpu_batch_phase_set", "agpu_phase_fetch", "agpu_batch_revise", "agpu_revise_fetch", "agpu_batch_upload_packed", "agpu_reserved", "agpu_reserve", "agpu_blocking_sync", "agpu_upload_async",
                "agpu_batch_results", "agpu_d2h_bytes", "agpu_pinned_match",
                "agpu_batch_group_support", "agpu_support_fetch", "agpu_batch_coverage_edit", "agpu_batch_preview", "agpu_preview_fetch",
-               "agpu_batch_gather", "agpu_batch_inputs"]
+               "agpu_batch_gather", "agpu_batch_inputs", "agpu_batch_group_phase_set", "agpu_group_phase_fetch"]
 
 
 def load(lib_path=None):
@@ -152,6 +152,8 @@ def load(lib_path=None):
     L.agpu_batch_bundle_counts.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
     L.agpu_batch_phase_set.argtypes = [C.c_void_p, C.c_void_p]
     L.agpu_phase_fetch.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(PhaseView)]
+    L.agpu_batch_group_phase_set.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
+    L.agpu_group_phase_fetch.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(PhaseView)]
     L.agpu_batch_revise.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(Params)]
     L.agpu_revise_fetch.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(ReviseView)]
     L.agpu_batch_group_bridge.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.POINTER(Params)]
@@ -513,15 +515,30 @@ class Batch:
     def phase_set(self):
         """bundle_base::build_phase_set against the current graphs; per bundle the oracle's phase_off / phase_val / phase_cnt"""
         self._run("phase_set")
+        return self._phase_view("agpu_phase_fetch", self.nb)
+
+    def group_phase_set(self, groups):
+        """the combined phase set px of every cluster (assembler::assemble(vector<bundle*>): px.combine(ps) over its members):
+        groups = list of lists of bundle indices, one member allowed; needs phase_set() first.  Per cluster the dict of
+        phase_set()"""
+        off = np.zeros(len(groups) + 1, np.int32)
+        for i, grp in enumerate(groups):
+            off[i + 1] = off[i] + len(grp)
+        mem = np.ascontiguousarray(np.concatenate([np.asarray(x, np.int32) for x in groups]) if groups else np.zeros(1, np.int32), np.int32)
+        self.ctx.check(self.ctx.L.agpu_batch_group_phase_set(self.ctx.h, self.h, len(groups), off.ctypes.data, mem.ctypes.data),
+                       "agpu_batch_group_phase_set")
+        return self._phase_view("agpu_group_phase_fetch", len(groups))
+
+    def _phase_view(self, fetch, n_seg):
         v = PhaseView()
-        self.ctx.check(self.ctx.L.agpu_phase_fetch(self.ctx.h, self.h, C.byref(v)), "agpu_phase_fetch")
-        nb, npz = self.nb, int(v.n_phases)
-        po = _arr(v.phase_off, nb + 1, np.int64)
+        self.ctx.check(getattr(self.ctx.L, fetch)(self.ctx.h, self.h, C.byref(v)), fetch)
+        npz = int(v.n_phases)
+        po = _arr(v.phase_off, n_seg + 1, np.int64)
         co = _arr(v.coord_off, npz + 1, np.int64)
         cv = _arr(v.coords, int(co[npz]) if npz else 0)
         cc = _arr(v.count, npz)
         out = []
-        for k in range(nb):
+        for k in range(n_seg):
             a, b = int(po[k]), int(po[k + 1])
             out.append({"phase_off": (co[a:b + 1] - co[a]).astype(np.int32), "phase_val": cv[int(co[a]):int(co[b])], "phase_cnt": cc[a:b]})
         return out

@@ -7,7 +7,8 @@ One sample per BAM.  The files are decoded on the host (host/bamio.cc), cut into
 meta/generator.cc:77-201), and cut by position into device batches (clusters.device_batches, include/aletsch_gpu.h, BATCHING
 RULE).  Without --clusters every device batch goes through bundle::bridge on its own.  With --clusters the bundles are clustered
 across samples (bundle_group::resolve per 1 Mb region and strand), regrouped on the device cluster by cluster, bridged, and every
-cluster is re-bridged against its combined splice graph (assembler::bridge): shard.cluster_pass_sharded.
+cluster is re-bridged against its combined splice graph (assembler::bridge) and given its combined phase set px:
+shard.cluster_pass_sharded (cluster_phases counts the distinct lists of all combined phase sets).
 
 Under torchrun (WORLD_SIZE > 1, one process per GPU, NCCL) the samples are sharded: rank r decodes the files with index
 i % world == r, and with --clusters every cluster's bundles are moved to one GPU for the cluster pass.  One process is the same
@@ -95,11 +96,12 @@ def _run(args, lt, rank, world, device):
     out = {"samples": len(recs), "bundles": batch.n_bundles, "decode_pack_s": t1 - t0, "device_batches": len(parts)}
     if args.clusters:
         srcs = [ctx.upload(p.view(), keepalive=p) for p in parts]
-        res = cluster_pass_sharded(ctx, parts, srcs, bundle_keys(batch), gp)
+        res = cluster_pass_sharded(ctx, parts, srcs, bundle_keys(batch), gp, phases=True)
         for s in srcs:
             s.free()
         out["region_groups"] = res.n_groups
         out["clusters_of_bundles"] = sum(len(c) for c in res.clusters)
+        out["cluster_phases"] = sum(len(px["phase_cnt"]) for b in res.phases for px in b)
         bts = res.batches
     else:
         def bridged(p):

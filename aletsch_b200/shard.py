@@ -254,7 +254,7 @@ def _exchange(ctx, batches, base, plan, g, rank, world, stats):
     return adopted
 
 
-def cluster_pass_sharded(ctx, parts, batches, keys, params, support=False, times=None):
+def cluster_pass_sharded(ctx, parts, batches, keys, params, support=False, times=None, phases=False):
     """clusters.cluster_pass for a job whose samples are ingested on different ranks (one process per GPU).
 
     parts / batches: this rank's host parts and device batches, as cluster_pass takes them; keys: the global key of every bundle
@@ -267,13 +267,14 @@ def cluster_pass_sharded(ctx, parts, batches, keys, params, support=False, times
     Returns a clusters.ClusterPass for this rank's clusters; its origin rows are (ingesting rank, global key, local part, index in
     the part), the last two -1 for a bundle received from another rank, and n_groups / n_clusters count the region groups and
     clusters of the whole job.  `.exchange` holds the bundles, hits and bytes this rank sent and received, and the bytes per peer
-    (bytes_to, bytes_from).  times: cluster_pass's phases.  Without a process group the result equals cluster_pass's."""
+    (bytes_to, bytes_from).  times: cluster_pass's phase times; phases: cluster_pass's combined phase sets, of this rank's
+    clusters.  Without a process group the result equals cluster_pass's."""
     grouped = dist.is_available() and dist.is_initialized()
     rank, world = (dist.get_rank(), dist.get_world_size()) if grouped else (0, 1)
-    return _cluster_pass(ctx, parts, batches, keys, params, support, times, rank, world)
+    return _cluster_pass(ctx, parts, batches, keys, params, support, times, rank, world, phases)
 
 
-def _cluster_pass(ctx, parts, batches, keys, params, support, times, rank, world):
+def _cluster_pass(ctx, parts, batches, keys, params, support, times, rank, world, phases=False):
     """the cross-sample cluster pass as rank `rank` of `world`; with world 1 nothing is communicated, whatever process group exists"""
     from .clusters import ClusterPass, _Clock, bundle_spans, run_clusters
     if len(parts) != len(batches):
@@ -285,6 +286,7 @@ def _cluster_pass(ctx, parts, batches, keys, params, support, times, rank, world
     clock = _Clock(ctx, batches, times)
     out = ClusterPass()
     out.support = [] if support else None
+    out.phases = [] if phases else None
     out.exchange = {k: 0 for k in ("bundles_sent", "hits_sent", "bytes_sent", "bundles_received", "hits_received", "bytes_received")}
     out.exchange.update(bytes_to=[0] * world, bytes_from=[0] * world)
     # 1. evidence on the sources, then bundle::splices of this rank's bundles
@@ -343,7 +345,7 @@ def _cluster_pass(ctx, parts, batches, keys, params, support, times, rank, world
     origin = np.stack([src_of, keys_all[rows], part, idx], axis=1).astype(np.int64)
     try:
         run_clusters(ctx, list(batches) + [adopted[d] for d in peers], picks, x[rows, 3], x[rows, 1], plan.cstart[rank], params, out,
-                     clock, support, origin)
+                     clock, support, origin, phases)
     finally:
         for b in adopted.values():
             b.free()

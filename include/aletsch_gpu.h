@@ -400,6 +400,19 @@ typedef struct agpu_phase_view
 int agpu_batch_phase_set(agpu_ctx *ctx, agpu_batch *b);
 int agpu_phase_fetch(agpu_ctx *ctx, agpu_batch *b, agpu_phase_view *v);
 
+/* ---- combined phase sets of bundle clusters: the `px` of assembler::assemble(vector<bundle*>) (meta/assembler.cc:177-373),
+ * which folds every member's phase set into one with px.combine(ps) right after bd.build_phase_set(ps, gr) and assembles the
+ * combined graph gx with it.  Cluster layout as agpu_batch_group_bridge (a cluster of one member is allowed: its px is its ps;
+ * a bundle may appear in at most one cluster).  px of a cluster is the union of its members' phase sets as agpu_phase_fetch
+ * lists them: equal coordinate lists become one entry whose count is the sum of theirs (phase_set::add,
+ * rnacore/phase_set.cc:12-25, for every entry of ps); the member order does not matter.  Call after agpu_batch_phase_set.
+ * AGPU_ERR_ARG (and no combined phase set afterwards) without a member phase set, for a bundle index out of range or a bundle
+ * listed twice; n_groups = 0 gives an empty view.  A later agpu_batch_phase_set, agpu_batch_group_bridge or agpu_batch_reset
+ * drops the combined phase sets; agpu_group_phase_fetch then returns AGPU_ERR_ARG.
+ * The view is agpu_phase_view with phase_off indexed by cluster [n_groups + 1]; every cluster's lists in phase_set::pmap order. */
+int agpu_batch_group_phase_set(agpu_ctx *ctx, agpu_batch *b, int32_t n_groups, const int32_t *group_off, const int32_t *group_bundles);
+int agpu_group_phase_fetch(agpu_ctx *ctx, agpu_batch *b, agpu_phase_view *v);
+
 /* ---- boundary revision: the revising half of assembler::transform(bd, gr, true) (meta/assembler.cc:930-944) on the bundles'
  * own splice graphs.  identify_boundaries (rnacore/graph_reviser.cc:1068-1283) adds a start edge 0 -> a / an end edge b -> n
  * wherever log(2 + maxcov) / log(2 + weight entering / leaving) of a continuous run of vertices reaches

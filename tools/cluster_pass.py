@@ -3,14 +3,19 @@
 
   python tools/cluster_pass.py --config 2                 the job cut by the batching rule (configs[2]: 4 device batches)
   python tools/cluster_pass.py --config 1 --cut 3 --check a forced 3-way cut, compared with the single-batch run
+  python tools/cluster_pass.py --config 1 --cut 3 --phases  with every cluster's combined phase set (px)
 
 Reports per phase the host-clock time around synchronised work after a warm-up pass (source evidence, stage 5, plan, gather, and per
 output batch bridge_all, group_bridge, group_support); the gather kernels' time from the per-kernel events (agpu_profile_enable),
 their algorithmic bytes (per hit 34 B read + 34 B written: 4 x i32, 2 x u8, u64 qid, u32 cigar_off; per CIGAR operation 4 B read + 4
 B written) and GB/s; the host route it replaces (PackedBatch.select + compact form + agpu_batch_upload_packed of the same output
 batches, from pageable host memory); and, with --check, the count of bundles whose digests (bench.view_digests) and of clusters whose
-support rows differ from the single-batch run.  Prints one JSON line; progress goes to stderr."""
+support rows differ from the single-batch run.  With --phases the pass also builds the combined phase sets, and per output batch
+the report gives the agpu_batch_group_phase_set and agpu_group_phase_fetch times (device synchronised, best of 3), the member lists
+going in (the distinct lists of every member's phase set) and the combined lists coming out, and the member agpu_phase_fetch time.
+Prints one JSON line; progress goes to stderr."""
 import argparse
+import ctypes as C
 import json
 import os
 import subprocess
@@ -48,10 +53,44 @@ def copy_peak():
         return 6543.1, "measured B200 copy peak named in BASELINE.md"
 
 
-def cluster_pass(ctx, parts, srcs, gp, support, times=None):
+def cluster_pass(ctx, parts, srcs, gp, support, times=None, phases=False):
     for s in srcs:
         s.reset()
-    return CL.cluster_pass(ctx, parts, srcs, gp, support=support, times=times)
+    return CL.cluster_pass(ctx, parts, srcs, gp, support=support, times=times, phases=phases)
+
+
+def best_of(f, reps=3):
+    dt = []
+    for _ in range(reps):
+        t0 = time.perf_counter()
+        f()
+        dt.append(time.perf_counter() - t0)
+    return min(dt)
+
+
+def phase_report(res):
+    """per output batch: group_phase_set / fetch seconds, lists in and out, member agpu_phase_fetch seconds (the pass left every
+    batch with its member phase sets and the combined ones)"""
+    rows = []
+    for bt, cl in zip(res.batches, res.clusters):
+        L, h = bt.ctx.L, bt.ctx.h
+        off = np.concatenate([[0], np.cumsum([len(c) for c in cl])]).astype(np.int32)
+        mem = np.ascontiguousarray(np.concatenate([np.asarray(c, np.int32) for c in cl]) if cl else np.zeros(1, np.int32))
+        v = G.PhaseView()
+
+        def build():
+            bt.ctx.check(L.agpu_batch_group_phase_set(h, bt.h, len(cl), off.ctypes.data, mem.ctypes.data), "agpu_batch_group_phase_set")
+            bt.ctx.sync()
+        t_build = best_of(build)
+        t_fetch = best_of(lambda: bt.ctx.check(L.agpu_group_phase_fetch(h, bt.h, C.byref(v)), "agpu_group_phase_fetch"))
+        t_member = best_of(lambda: bt.ctx.check(L.agpu_phase_fetch(h, bt.h, C.byref(v)), "agpu_phase_fetch"))
+        po = G._arr(v.phase_off, bt.nb + 1, np.int64)
+        lists_in = int(sum(int(po[m + 1] - po[m]) for c in cl for m in c))
+        lists_out = int(sum(len(px["phase_cnt"]) for px in res.phases[len(rows)]))
+        rows.append({"clusters": len(cl), "group_phase_set_s": round(t_build, 5), "group_phase_fetch_s": round(t_fetch, 5),
+                     "lists_in": lists_in, "lists_out": lists_out, "member_phase_fetch_s": round(t_member, 5),
+                     "member_lists": int(v.n_phases)})
+    return rows
 
 
 def single_batch(ctx, batch, gp, support):
@@ -98,6 +137,7 @@ def main():
     ap.add_argument("--cut", type=int, default=0, help="cut the job into this many parts instead of by the batching rule")
     ap.add_argument("--check", action="store_true", help="compare with the single-batch run (the job must fit one device batch)")
     ap.add_argument("--no-support", action="store_true")
+    ap.add_argument("--phases", action="store_true", help="also the combined phase set of every cluster (phases=True)")
     args = ap.parse_args()
     support = not args.no_support
     cfg = bench.config_of(args)
@@ -118,12 +158,14 @@ def main():
         per_bundle_bridged += int(s.bundle_counts()[:, 3].sum())
 
     bench.log("[cluster_pass] warm-up pass")
-    cluster_pass(ctx, parts, srcs, gp, support).free()
+    cluster_pass(ctx, parts, srcs, gp, support, phases=args.phases).free()
     bench.log("[cluster_pass] timed pass")
     times = {}
     t0 = time.perf_counter()
-    res = cluster_pass(ctx, parts, srcs, gp, support, times)
+    res = cluster_pass(ctx, parts, srcs, gp, support, times, phases=args.phases)
     total_s = time.perf_counter() - t0
+    if args.phases:
+        out["phases"] = phase_report(res)
     multi = [c for cl in res.clusters for c in cl]
     bridged = int(sum(int(b.bundle_counts()[:, 3].sum()) for b in res.batches))
     cnt = [b.counts() for b in res.batches]
