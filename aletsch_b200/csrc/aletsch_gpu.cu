@@ -237,8 +237,9 @@ static int check_err(agpu_ctx *ctx, agpu_batch *b, const char *stage)
 	TRY(d2h(ctx, e, b->err.p, sizeof(e)));
 	TRY(stream_sync(ctx));
 	const char *names[] = {"hit order", "duplicate (pos,rpos)", "mixed strand", "rpos != pos + cigar2rlen", "junction without partial exon",
-		"reserved qid", "scratch capacity", "compact input without the escape entry a sentinel announces"};
-	for(int k = 0; k < 8; k++)
+		"reserved qid", "scratch capacity", "compact input without the escape entry a sentinel announces",
+		"two partial exons with a common bound"};
+	for(int k = 0; k <= ERR_BOUNDS; k++)
 	{
 		if(e[k] == 0) continue;
 		char buf[256];

@@ -39,7 +39,7 @@ struct hits_dev
 };
 
 // error / statistics words shared by all kernels of a batch
-enum { ERR_ORDER = 0, ERR_DUP, ERR_STRAND, ERR_RPOS, ERR_LINK, ERR_QID, ERR_CAP, ERR_PACKED, ERR_WORDS = 16 };
+enum { ERR_ORDER = 0, ERR_DUP, ERR_STRAND, ERR_RPOS, ERR_LINK, ERR_QID, ERR_CAP, ERR_PACKED, ERR_BOUNDS, ERR_WORDS = 16 };
 
 // ---- E0: bundle bounds (bundle_base::add_hit) + packing-contract check.  One thread per HIT (bundles range from one hit to
 // several hundred thousand: a CTA per bundle leaves the step waiting for the deepest one).  A hit finds its bundle by bisection of

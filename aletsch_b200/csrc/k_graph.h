@@ -545,7 +545,12 @@ KERNEL k_graph_build(const int32_t *order, int n_order, graph_in in, graph_dev g
 		}
 		BLOCK_SYNC();
 
-		// ---- link junctions to partial exons (rnacore/graph_builder.cc:244-297)
+		// ---- link junctions to partial exons (rnacore/graph_builder.cc:244-297).  The reference asserts that no two partial
+		// exons share an lpos or an rpos (:255-258).  Only a 1-bp region between a junction end and a junction start, uncovered
+		// and not smoothed (min_subregion_gap 0), breaks that: it gets both stubs, [p, p + 1) twice.  Partial exons are in
+		// position order, so such a pair is adjacent; it is reported like a missing exon (AGPU_ERR_INPUT).
+		for(int i = t + 1; i < np; i += nt)
+			if(g.p_l[p0 + i] == g.p_l[p0 + i - 1] || g.p_r[p0 + i] == g.p_r[p0 + i - 1]) atomicAdd(&g.err[ERR_BOUNDS], 1);
 		int32_t *jout = ia; ia += np + 2;              // junction out-degree of pexon i
 		int32_t *jin = ia; ia += np + 2;
 		for(int i = t; i < np + 2; i += nt) { jout[i] = 0; jin[i] = 0; }

@@ -322,6 +322,21 @@ class Context:
         self.check(self.L.agpu_similarity(self.h, g, off.ctypes.data, val.ctypes.data, c.ctypes.data, r.ctypes.data), "agpu_similarity")
         return c, r
 
+    def similarity_batch(self, groups):
+        """agpu_similarity_batch: groups is a list of lists of sorted splice lists; returns one dense G x G int32 matrix of
+        |A∩B| per group (the pairs i < j are filled)"""
+        flat = [l for grp in groups for l in grp]
+        off, val = _pack_lists(flat)
+        goff = np.zeros(len(groups) + 1, np.int32)
+        coff = np.zeros(len(groups) + 1, np.int64)
+        for i, grp in enumerate(groups):
+            goff[i + 1] = goff[i] + len(grp)
+            coff[i + 1] = coff[i] + len(grp) * len(grp)
+        c = np.zeros(max(int(coff[-1]), 1), np.int32)
+        self.check(self.L.agpu_similarity_batch(self.h, len(groups), goff.ctypes.data, off.ctypes.data, val.ctypes.data,
+                                                coff.ctypes.data, c.ctypes.data), "agpu_similarity_batch")
+        return [c[int(coff[i]):int(coff[i + 1])].reshape(len(grp), len(grp)) for i, grp in enumerate(groups)]
+
 
 def _pack_lists(lists):
     g = len(lists)

@@ -69,6 +69,7 @@ typedef struct orc_params
 	double min_grouping_similarity;
 	double max_grouping_similarity;
 	double min_boundary_log_ratio;
+	int32_t max_group_boundary_distance;  /* appended like agpu_params: the layouts stay equal */
 } orc_params;
 
 /* result bag: named flat arrays, kind 0 = int32, 1 = float64 */
@@ -92,6 +93,10 @@ const void *orc_bag_data(void *bag, int i);
 	int P##_bundle_revise(void *b, void *bag); \
 	int P##_group_bridge(void **bs, int n, void *bag); \
 	int P##_group_resolve(void **bs, int n, const orc_params *prm, void *bag);
+
+/* restatement only: <P>_group_resolve on n given sorted splice lists (list k = list_val[list_off[k] .. list_off[k + 1])) instead of
+ * bundle handles, so that constructed lists can be checked; "gvv_off" / "gvv_val" as there */
+int orc_group_resolve_lists(int n, const int64_t *list_off, const int32_t *list_val, const orc_params *prm, void *bag);
 
 /* reference build only: generator::resolve (meta/generator.cc:51-227) over the records served through the htslib stand-in;
  * dumps the bundles it creates (gen_off, gen_bundle = tid lpos rpos strand per bundle, gen_pos / rpos / mpos / isize / flag /

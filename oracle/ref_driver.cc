@@ -69,6 +69,7 @@ void apply_params(const orc_params *p, parameters &cfg, sample_profile &sp)
 	cfg.min_grouping_similarity = p->min_grouping_similarity;
 	cfg.max_grouping_similarity = p->max_grouping_similarity;
 	cfg.min_boundary_log_ratio = p->min_boundary_log_ratio;
+	cfg.max_group_boundary_distance = p->max_group_boundary_distance;
 	sp.library_type = p->library_type;
 	sp.insertsize_low = p->insertsize_low;
 	sp.insertsize_high = p->insertsize_high;

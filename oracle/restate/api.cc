@@ -243,7 +243,7 @@ int orc_bundle_graph(void *b, void *bagp)
 	build_graph(bd, gr, bo);
 	dump_builder(bo, bag, "");
 	dump_graph(gr, bag, "");
-	return 0;
+	return bo.repeated_bounds ? -1 : 0;            // where the reference asserts
 }
 
 // bundle::bridge (meta/bundle.cc:55-88)
@@ -254,6 +254,7 @@ int orc_bundle_bridge(void *b, void *bagp)
 	graph gr;
 	builder_out bo;
 	build_graph(bd, gr, bo);
+	if(bo.repeated_bounds) return -1;                 // where the reference asserts (see builder_out)
 	dump_builder(bo, bag, "");
 	dump_graph(gr, bag, "");
 	return cluster_solve_update(gr, bd, bd.prm, bag, "", false);
@@ -267,6 +268,7 @@ int orc_bundle_phase(void *b, void *bagp)
 	graph gr;
 	builder_out bo;
 	build_graph(bd, gr, bo);
+	if(bo.repeated_bounds) return -1;                 // where the reference asserts (see builder_out)
 	std::map<chain_t, int> ps;
 	build_phase_set(bd, gr, ps);
 	std::vector<int32_t> &po = bag.ints("phase_off");
@@ -291,6 +293,7 @@ int orc_bundle_revise(void *b, void *bagp)
 	graph gr;
 	builder_out bo;
 	build_graph(bd, gr, bo);
+	if(bo.repeated_bounds) return -1;                 // where the reference asserts (see builder_out)
 	revision rv;
 	revise_graph(bd, gr, rv);
 	std::vector<int32_t> &re = bag.ints("rev_edge");
@@ -348,7 +351,7 @@ int orc_group_support(void **bs, int n, void *bagp)
 	std::vector<support> sups;
 	graph gx;
 	support sx;
-	group_support((bundle**)bs, n, grs, sups, gx, sx);
+	if(group_support((bundle**)bs, n, grs, sups, gx, sx)) return -1;
 	for(int k = 0; k < n; k++)
 	{
 		char pre[32];
@@ -392,6 +395,7 @@ int orc_group_bridge(void **bs, int n, void *bagp)
 	graph gr;
 	builder_out bo;
 	build_graph(cb, gr, bo);
+	if(bo.repeated_bounds) return -1;                 // where the reference asserts (see builder_out)
 	dump_builder(bo, bag, "cb_");
 	dump_graph(gr, bag, "cb_");
 	int total = 0;
@@ -404,12 +408,12 @@ int orc_group_bridge(void **bs, int n, void *bagp)
 	return total;
 }
 
-// bundle_group::resolve (meta/bundle_group.cc:26-56) on the bundles' splice lists
-int orc_group_resolve(void **bs, int n, const orc_params *prm, void *bagp)
+namespace {
+
+// bundle_group::resolve (meta/bundle_group.cc:26-56) on n sorted splice lists
+int resolve_lists(const std::vector<const std::vector<int32_t>*> &sp, const orc_params *prm, orc_bag &bag)
 {
-	orc_bag &bag = *(orc_bag*)bagp;
-	std::vector<const std::vector<int32_t>*> sp(n);
-	for(int k = 0; k < n; k++) sp[k] = &((bundle*)bs[k])->splices;
+	const int n = (int)sp.size();
 	// build_splice_index (:150-172)
 	std::map<int32_t, std::set<int> > sindex;
 	for(int k = 0; k < n; k++) for(size_t i = 0; i < sp[k]->size(); i++) sindex[(*sp[k])[i]].insert(k);
@@ -483,6 +487,29 @@ int orc_group_resolve(void **bs, int n, const orc_params *prm, void *bagp)
 	off.assign(1, 0); val.clear();
 	for(size_t i = 0; i < gvv.size(); i++) { val.insert(val.end(), gvv[i].begin(), gvv[i].end()); off.push_back((int32_t)val.size()); }
 	return 0;
+}
+
+} // namespace
+
+// bundle_group::resolve on the bundles' splice lists
+int orc_group_resolve(void **bs, int n, const orc_params *prm, void *bagp)
+{
+	std::vector<const std::vector<int32_t>*> sp(n);
+	for(int k = 0; k < n; k++) sp[k] = &((bundle*)bs[k])->splices;
+	return resolve_lists(sp, prm, *(orc_bag*)bagp);
+}
+
+// the same on given lists: list k is list_val[list_off[k] .. list_off[k + 1])
+int orc_group_resolve_lists(int n, const int64_t *list_off, const int32_t *list_val, const orc_params *prm, void *bagp)
+{
+	std::vector<std::vector<int32_t> > lists(n);
+	std::vector<const std::vector<int32_t>*> sp(n);
+	for(int k = 0; k < n; k++)
+	{
+		lists[k].assign(list_val + list_off[k], list_val + list_off[k + 1]);
+		sp[k] = &lists[k];
+	}
+	return resolve_lists(sp, prm, *(orc_bag*)bagp);
 }
 
 

@@ -380,9 +380,16 @@ void build_graph(const bundle &bd, graph &gr, builder_out &bo)
 		pe.pvalue = b ? 0 : 1;
 	}
 
-	// link_partial_exons (:244-297)
+	// link_partial_exons (:244-297): the reference asserts that no two partial exons share a bound (:255-258) before it
+	// inserts them into its maps; a 1-bp region between a junction end and a junction start with no coverage and
+	// min_subregion_gap 0 gets both stubs of build_partial_exons, [p, p + 1) twice
 	std::map<int32_t, int> lm, rm;
-	for(size_t i = 0; i < pexons.size(); i++) { lm[pexons[i].lpos] = (int)i; rm[pexons[i].rpos] = (int)i; }
+	bo.repeated_bounds = 0;
+	for(size_t i = 0; i < pexons.size(); i++)
+	{
+		if(!lm.insert(std::make_pair(pexons[i].lpos, (int)i)).second) bo.repeated_bounds++;
+		if(!rm.insert(std::make_pair(pexons[i].rpos, (int)i)).second) bo.repeated_bounds++;
+	}
 	for(size_t i = 0; i < junctions.size(); i++)
 	{
 		std::map<int32_t, int>::iterator li = rm.find(junctions[i].lpos), ri = lm.find(junctions[i].rpos);

@@ -115,7 +115,9 @@ struct revision
 	std::vector<double> leave_ratio, come_ratio;
 };
 
-struct builder_out { std::vector<junction> junctions; std::vector<pexon> pexons; };
+// repeated_bounds: partial exons whose lpos or rpos an earlier one already has; link_partial_exons asserts there are none
+// (rnacore/graph_builder.cc:255-258), so the graph is not the reference's when this is non-zero
+struct builder_out { std::vector<junction> junctions; std::vector<pexon> pexons; int repeated_bounds = 0; };
 
 void build_graph(const bundle &bd, graph &gr, builder_out &bo);
 void build_phase_set(const bundle &bd, const graph &gr, std::map<chain_t, int> &ps);
@@ -132,7 +134,8 @@ struct support
 	std::vector<std::array<double, 4> > loss;           // boundary_loss1, 2, 3, boundary_merged_loss per vertex
 };
 // one entry per member in grs / sups: the state at the point where the reference assembles that member
-void group_support(bundle **bs, int n, std::vector<graph> &grs, std::vector<support> &sups, graph &gx, support &sx);
+// returns -1 (and leaves the outputs partial) if a graph it builds has repeated partial-exon bounds
+int group_support(bundle **bs, int n, std::vector<graph> &grs, std::vector<support> &sups, graph &gx, support &sx);
 void build_fragments(bundle &bd);
 void cluster_fragments(graph &gr, bundle &bd, std::vector<cluster> &vc);
 void bridge_clusters(graph &gr, std::vector<cluster> &vc, const orc_params &prm, std::vector<bridge_path> &opt);

@@ -265,12 +265,13 @@ static void group_boundaries(graph &gr, int32_t max_dist)
 	}
 }
 
-void group_support(bundle **bs, int n, std::vector<graph> &grs, std::vector<support> &sups, graph &gx, support &sx)
+int group_support(bundle **bs, int n, std::vector<graph> &grs, std::vector<support> &sups, graph &gx, support &sx)
 {
 	bundle cb;
 	combine_bundles(bs, n, cb, NULL);
 	builder_out bo;
 	build_graph(cb, gx, bo);
+	if(bo.repeated_bounds) return -1;
 	std::map<junc_key, junc_val> jm;
 	init_support(gx, sx, -1, jm);
 	std::vector<graph> live(n);                           // the graphs as the rounds see them (regrouped once assembled)
@@ -279,6 +280,7 @@ void group_support(bundle **bs, int n, std::vector<graph> &grs, std::vector<supp
 	{
 		builder_out bk;
 		build_graph(*bs[k], live[k], bk);
+		if(bk.repeated_bounds) return -1;
 		revision rv;
 		revise_graph(*bs[k], live[k], rv);
 		init_support(live[k], sups[k], bs[k]->sample, jm);
@@ -296,9 +298,10 @@ void group_support(bundle **bs, int n, std::vector<graph> &grs, std::vector<supp
 		non_splicing_support(bs[k]->sample, live[k], gx, sx);
 		boundary_extend(-1, live[k], sups[k], gx, 1);
 		grs[k] = live[k];                                 // what the reference hands to assemble(gr, ps, sid) ...
-		group_boundaries(live[k], 10000);                 // ... which regroups its boundaries (max_group_boundary_distance, util/parameters.cc:77)
+		group_boundaries(live[k], bs[0]->prm.max_group_boundary_distance);   // ... which regroups its boundaries (util/parameters.cc:77)
 	}
 	junction_support(gx, sx, jm);
+	return 0;
 }
 
 } // namespace orc

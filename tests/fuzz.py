@@ -170,3 +170,63 @@ def strand_clusters(batch, rng):
             groups.append([int(x) for x in ks[:n]])
             ks = ks[n:]
     return groups
+
+
+def dag_bundle(n_exons, reads_per_junction=1, strand="+", pairs=3, exon_len=20, step=100, base=1000):
+    """one bundle whose splice graph is a complete DAG: n_exons exons of exon_len bases, a junction from every exon to every
+    later one (reads_per_junction + (i + j) % 3 spliced reads each, so the weights differ), and `pairs` read pairs with one
+    mate in the first exon and the other in the last.  Every pair is one cluster whose bridging range holds all exons, so the
+    bridging DP of the last exons sees up to K candidates from each earlier exon."""
+    X = [base + step * i for i in range(n_exons)]
+    hits = []        # (pos, cigar ops, qid, mpos, isize, flag)
+    q = 1
+    for i in range(n_exons):
+        for j in range(i + 1, n_exons):
+            for r in range(reads_per_junction + (i + j) % 3):
+                a = exon_len // 2 + r % (exon_len // 2 - 1)       # the read starts a bases into exon i
+                p = X[i] + a
+                ops = [(M, exon_len - a), (N, X[j] - X[i] - exon_len), (M, 3 + r % 5)]
+                hits.append((p, ops, q, 0, 0, 0))
+                q += 1
+    for k in range(pairs):
+        p1, p2 = X[0] + k, X[-1] + 1 + k
+        sz = p2 + 12 - p1
+        hits.append((p1, [(M, 12)], q, p2, sz, 0x1 | 0x2 | 0x20 | 0x40))
+        hits.append((p2, [(M, 12)], q, p1, -sz, 0x1 | 0x2 | 0x10 | 0x80))
+        q += 1
+    hits.sort(key=lambda h: (h[0], sum(l for o, l in h[1] if o in REF_OPS)))
+    out = {"pos": np.array([h[0] for h in hits], np.int32)}
+    cig, co, rp = [], [0], []
+    for h in hits:
+        cig.extend((l << 4) | o for o, l in h[1])
+        co.append(len(cig))
+        rp.append(h[0] + sum(l for o, l in h[1] if o in REF_OPS))
+    out["rpos"] = np.array(rp, np.int32)
+    out["cigar"] = np.array(cig, np.uint32)
+    out["cigar_off"] = np.array(co, np.uint32)
+    out["qid"] = np.array([h[2] for h in hits], np.uint64)
+    out["mpos"] = np.array([h[3] for h in hits], np.int32)
+    out["isize"] = np.array([h[4] for h in hits], np.int32)
+    out["flag"] = np.array([h[5] for h in hits], np.uint16)
+    out["strand"] = np.full(len(hits), ord(strand), np.uint8)
+    out["xs"] = np.array([ord(strand) if len(h[1]) > 1 else ord(".") for h in hits], np.uint8)
+    return out
+
+
+def pack_bundles(parts):
+    """a PackedBatch of bundles given as dicts of hit arrays (as random_bundle returns them)"""
+    arr = {f: (np.concatenate([p[f] for p in parts]).astype(dt) if parts else np.zeros(0, dt)) for f, dt in H.HIT_FIELDS}
+    hit_off = np.zeros(len(parts) + 1, np.int64)
+    cig_off = [np.zeros(1, np.uint32)]
+    cbase = 0
+    for i, p in enumerate(parts):
+        hit_off[i + 1] = hit_off[i] + len(p["pos"])
+        cig_off.append(p["cigar_off"][1:] + np.uint32(cbase))
+        cbase += len(p["cigar"])
+    arr["bundle_hit_off"] = hit_off
+    arr["cigar_off"] = np.concatenate(cig_off).astype(np.uint32)
+    arr["cigar"] = np.concatenate([p["cigar"] for p in parts]).astype(np.uint32) if parts else np.zeros(0, np.uint32)
+    arr["bundle_tid"] = np.zeros(len(parts), np.int32)
+    arr["bundle_sample"] = np.zeros(len(parts), np.int32)
+    arr["bundle_side"] = np.zeros(len(parts), np.uint8)
+    return H.PackedBatch(arr)

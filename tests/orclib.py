@@ -23,7 +23,7 @@ class Params(C.Structure):
                 ("insertsize_high", C.c_int32), ("max_group_size", C.c_int32), ("max_num_junctions_to_combine", C.c_int32),
                 ("min_subregion_overlap", C.c_double), ("min_guaranteed_edge_weight", C.c_double),
                 ("min_grouping_similarity", C.c_double), ("max_grouping_similarity", C.c_double),
-                ("min_boundary_log_ratio", C.c_double)]
+                ("min_boundary_log_ratio", C.c_double), ("max_group_boundary_distance", C.c_int32)]
 
 
 def default_params(**kw):
@@ -32,7 +32,8 @@ def default_params(**kw):
                min_subregion_gap=15, min_subregion_length=15, max_reads_partition_gap=10, bridge_end_relaxing=10,
                bridge_dp_solution_size=10, bridge_dp_stack_size=5, insertsize_low=80, insertsize_high=500,
                max_group_size=200, max_num_junctions_to_combine=500, min_subregion_overlap=1.5,
-               min_guaranteed_edge_weight=0.01, min_grouping_similarity=0.10, max_grouping_similarity=0.80, min_boundary_log_ratio=2.0)
+               min_guaranteed_edge_weight=0.01, min_grouping_similarity=0.10, max_grouping_similarity=0.80, min_boundary_log_ratio=2.0,
+               max_group_boundary_distance=10000)
     for k, v in kw.items():
         setattr(p, k, v)
     return p
